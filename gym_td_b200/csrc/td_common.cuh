@@ -99,7 +99,8 @@ struct DevConfig {
     double destruct_return, frozen_ratio, atk_init_cost, def_init_cost, max_cost;
     double reward_kill, penalty_leak, reward_time, rate_init, rate_final, def_rate, upgrade_at;
     int frozen_time, base_LP, tower_distance, atk_interval, def_interval, max_steps;
-    int upgrade_step;       // smallest s with (double)s / max_steps >= enemy_upgrade_at (TDBoard.py:201 without the division)
+    int upgrade_step;       // smallest s with (double)s / max_steps >= enemy_upgrade_at (TDBoard.py:201 without the division),
+                            // INT_MAX when no step count below INT_MAX reaches it (td_upgrade_step)
     double min_enemy_cost[TD_NLV];   // cheapest enemy type per level: below it every remaining cluster slot fails
 };
 

@@ -7,6 +7,7 @@
 #include <cuda.h>          // driver API types only: entry points are resolved at run time (no libcuda link dependency)
 
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -142,6 +143,24 @@ static int validate_config(td_handle *h, const td_config *c)
     return TD_OK;
 }
 
+// progress = steps / max_steps is monotone in steps (correctly rounded division of exact integers), so the first
+// step count whose f64 quotient reaches the threshold decides the enemy level exactly like
+// `self.progress >= config.enemy_upgrade_at` does, for every step count, also past the end of the episode.
+// ceil(at * max) is within a few counts of it; the two walks land on the first count that passes the test itself.
+extern "C" int td_upgrade_step(int max_episode_steps, double enemy_upgrade_at)
+{
+    const int kNever = 0x7fffffff;
+    if (max_episode_steps < 1) return kNever;
+    const double m = (double)max_episode_steps, at = enemy_upgrade_at;
+    if (!(at > 0.0)) return at <= 0.0 ? 0 : kNever;            // 0 / max >= at; NaN never compares true
+    auto reaches = [m, at](long long s) { volatile double q = (double)s / m; return q >= at; };
+    const double guess = std::ceil(at * m);
+    long long s = guess < (double)kNever ? (long long)guess : (long long)kNever;
+    while (s > 0 && reaches(s - 1)) --s;
+    while (s < kNever && !reaches(s)) ++s;
+    return (int)s;
+}
+
 // td_config -> the derived tables the kernels read.  The result lives in the handle and rides in the kernel
 // parameters of every launch, so handles with different configs coexist on one device.
 static int derive_config(td_handle *h, const td_config *c)
@@ -180,13 +199,7 @@ static int derive_config(td_handle *h, const td_config *c)
     d.rate_final = c->attacker_cost_final_rate;
     d.def_rate = c->defender_cost_rate;
     d.upgrade_at = c->enemy_upgrade_at;
-    // progress = steps / max_steps is monotone in steps: the first step count whose f64 quotient reaches the
-    // threshold decides the enemy level exactly like `self.progress >= config.enemy_upgrade_at` does
-    d.upgrade_step = 0x7fffffff;
-    for (int sidx = 0; sidx <= c->max_episode_steps + 1; ++sidx) {
-        volatile double prog = (double)sidx / (double)c->max_episode_steps;
-        if (prog >= c->enemy_upgrade_at) { d.upgrade_step = sidx; break; }
-    }
+    d.upgrade_step = td_upgrade_step(c->max_episode_steps, c->enemy_upgrade_at);
     for (int lv = 0; lv < TD_NLV; ++lv) {
         d.min_enemy_cost[lv] = d.enemy_cost[0][lv];
         for (int t = 1; t < TD_NTYPES; ++t) d.min_enemy_cost[lv] = std::min(d.min_enemy_cost[lv], d.enemy_cost[t][lv]);

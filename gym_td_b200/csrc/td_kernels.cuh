@@ -218,7 +218,11 @@ __device__ __forceinline__ void env_rules(const StepParams &p, const int env, W 
         h->ep_return = __dadd_rn(h->ep_return, reward);
         h->ep_kills = (uint16_t)(h->ep_kills + kills);
         h->ep_leaks = (uint16_t)(h->ep_leaks + leaks);
-        if (done) {
+        // An episode counts once, on the step where it ends.  A finished env that is stepped on without a reset
+        // (auto_reset off; the reference has no done latch) reports done again: the header in the slice still holds
+        // the pre-step base_LP / steps, and an env that had already ended before this step is not counted again.
+        const bool ended_before = h->steps > 0 && ((has_base && h->base_LP <= 0) || h->steps >= cc.max_steps);
+        if (done && !ended_before) {
             EnvStats &s = p.stats[env];
             s.return_sum = __dadd_rn(s.return_sum, h->ep_return);
             s.episodes += 1;

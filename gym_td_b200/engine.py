@@ -96,7 +96,7 @@ EXPORTS = ["td_abi_version", "td_last_error", "td_default_config", "td_mapgen", 
            "td_seed_opponent", "td_set_difficulty", "td_step", "td_observe", "td_step_host", "td_get_state",
            "td_set_state", "td_get_opponent", "td_get_stats", "td_reset_stats", "td_rollout_mask", "td_rollout_record",
            "td_gae", "td_snapshot", "td_observe_snapshot", "td_set_option", "td_packed_stride", "td_invalidate_obs", "td_observe_as",
-           "td_alloc_compressible", "td_free_compressible"]
+           "td_alloc_compressible", "td_free_compressible", "td_upgrade_step"]
 
 
 def lib():
@@ -143,6 +143,7 @@ def lib():
         L.td_observe_as.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         L.td_alloc_compressible.argtypes = [C.c_int, C.c_size_t, C.c_void_p, C.c_void_p]
         L.td_free_compressible.argtypes = [C.c_void_p]
+        L.td_upgrade_step.argtypes = [C.c_int, C.c_double]
         if L.td_abi_version() != 3:
             raise ImportError("libtd_b200.so ABI version mismatch")
         _lib = L
@@ -175,6 +176,25 @@ class CompressibleBuffer:
             _lib.td_free_compressible(C.c_void_p(ptr))
 
 
+def _base_lp(v):
+    """base_LP -> the td_config field (-1: no base).  The reference compares the live count with `<= 0`, so a
+    fraction would add a leak (5.5 ends after 6 leaks) and a negative count would end every step: both rejected."""
+    if v is None:
+        return -1
+    try:
+        iv = int(v)
+    except (TypeError, ValueError, OverflowError):
+        raise ValueError("base_LP must be None or a non-negative integer, got %r" % (v,))
+    if iv != v or iv < 0:
+        raise ValueError("base_LP must be None or a non-negative integer, got %r" % (v,))
+    return iv
+
+
+def upgrade_step(max_episode_steps, enemy_upgrade_at):
+    """First step count from which summoned enemies are level 1 (td_upgrade_step; 2**31 - 1: never)."""
+    return lib().td_upgrade_step(int(max_episode_steps), float(enemy_upgrade_at))
+
+
 def config_struct(cfg=None, hyper=None):
     """Snapshot a reference-style config object / dict into a td_config."""
     cfg = params.config if cfg is None else cfg
@@ -196,7 +216,7 @@ def config_struct(cfg=None, hyper=None):
         if name in d and name not in ("base_LP", "pad_"):
             setattr(c, name, d[name])
     if "base_LP" in d:
-        c.base_LP = -1 if d["base_LP"] is None else int(d["base_LP"])
+        c.base_LP = _base_lp(d["base_LP"])
     c.max_episode_steps = int(hyper.get("max_episode_steps", 1200))
     return c
 

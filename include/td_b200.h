@@ -239,6 +239,9 @@ typedef struct td_stats {
 int td_abi_version(void);
 const char *td_last_error(const td_handle *h);
 void td_default_config(td_config *cfg);
+/* host-only: the first step count s with (double)s / max_episode_steps >= enemy_upgrade_at, from which summoned
+ * enemies are level 1 (also past the end of an episode); 0x7fffffff when no smaller count reaches it (NaN, huge) */
+int td_upgrade_step(int max_episode_steps, double enemy_upgrade_at);
 
 /* host-only: reference-order road generator on a NumPy-legacy MT19937 stream.
  * num_roads <= 0: draw it first from the same stream like TDGymBasic.reset (:42).

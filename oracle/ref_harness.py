@@ -25,6 +25,15 @@ def set_multiple_actions(flag):
     hyper_parameters.__dict__["allow_multiple_actions"] = bool(flag)
 
 
+def set_max_episode_steps(n):
+    """hyper_parameters.max_episode_steps, poked like allow_multiple_actions; returns the previous value."""
+    ref_loader.load()
+    from gym_TD.envs.TDParam import hyper_parameters
+    old = hyper_parameters.__dict__["max_episode_steps"]
+    hyper_parameters.__dict__["max_episode_steps"] = int(n)
+    return old
+
+
 def ref_config():
     ref_loader.load()
     from gym_TD.envs.TDParam import config

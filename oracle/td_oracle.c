@@ -253,6 +253,7 @@ int tdo_summon_enemy(tdo_env *e, int t, int start_id)
     if (e->cost_atk < en.cost) { e->fail_code = TDO_COST_SHORTAGE; return 0; }
     en.uid = e->next_uid++;
     e->enemies[e->n_enemies++] = en;
+    if (e->n_enemies > e->peak_enemies) e->peak_enemies = e->n_enemies;
     e->cost_atk -= en.cost;
     e->fail_code = TDO_SUCCESS;
     return 1;
@@ -276,6 +277,7 @@ int tdo_summon_cluster(tdo_env *e, const int64_t *types, int start_id, int64_t *
             e->cost_atk -= en.cost;
             en.uid = e->next_uid++;
             e->enemies[e->n_enemies++] = en;
+            if (e->n_enemies > e->peak_enemies) e->peak_enemies = e->n_enemies;
             summoned = 1;
             if (real_act) real_act[k] = t;
         }
@@ -311,6 +313,7 @@ int tdo_tower_build(tdo_env *e, int t, int loc)
     if (e->cost_def < p.cost) { e->fail_code = TDO_COST_SHORTAGE; return 0; }
     if (e->map6[loc] > 0) { e->fail_code = TDO_INVALID_POSITION; return 0; }
     e->towers[e->n_towers++] = p;
+    if (e->n_towers > e->peak_towers) e->peak_towers = e->n_towers;
     e->cost_def -= p.cost;
     diamond_add(e, loc, +1);
     e->fail_code = TDO_SUCCESS;

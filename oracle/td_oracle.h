@@ -107,6 +107,8 @@ typedef struct tdo_env {
     tdo_mt nprand;   /* self.np_random */
     /* per-step counters (not in the reference; for statistics parity) */
     int32_t last_kills, last_leaks;
+    /* longest tower / enemy list since the caller last set these (not in the reference; for the capacity tests) */
+    int32_t peak_towers, peak_enemies;
 } tdo_env;
 
 /* outputs of one env-wrapper step: (obs,) reward, done, info */

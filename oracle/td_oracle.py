@@ -72,6 +72,7 @@ class Env(C.Structure):
         ("enemy_LP", ((C.c_float * MAX_CELLS) * NT) * 4),
         ("pyrand", MT), ("nprand", MT),
         ("last_kills", C.c_int32), ("last_leaks", C.c_int32),
+        ("peak_towers", C.c_int32), ("peak_enemies", C.c_int32),
     ]
 
 

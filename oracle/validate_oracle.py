@@ -42,7 +42,19 @@ def check_step(tag, env, o, obs_ref, rew_ref, done_ref, out, rew_or, step):
         raise AssertionError("%s step %d mismatch: %s" % (tag, step, bad))
 
 
-def run_def(L, seed, rs, difficulty=1, random_agent=True, max_steps=1200, multi=False):
+def _episode_over(done, left):
+    """True where a run stops: at the first `done`, or left[0] steps after it (the reference has no done latch, so a
+    finished env keeps stepping).  left = [steps after done, ended]."""
+    left[1] = left[1] or bool(done)
+    if not left[1]:
+        return False
+    if left[0] == 0:
+        return True
+    left[0] -= 1
+    return False
+
+
+def run_def(L, seed, rs, difficulty=1, random_agent=True, max_steps=1200, multi=False, past_done=0):
     seed, env = RH.first_valid_seed("def", L, seed, difficulty=difficulty, random_agent=random_agent)
     o = oracle_from_ref_env(env, current_oracle_config())
     random.seed(seed)
@@ -51,6 +63,7 @@ def run_def(L, seed, rs, difficulty=1, random_agent=True, max_steps=1200, multi=
     tag = "def L=%d seed=%d diff=%d ra=%s multi=%s" % (L, seed, difficulty, random_agent, multi)
     assert np.array_equal(env._board.get_states(), o.get_states()), tag + " obs0"
     nop = 6 * L * L
+    left = [past_done, False]
     for step in range(1, max_steps + 1):
         if multi:
             a = RH.sparse_multi_action(env._board, rs, p=0.02)
@@ -66,17 +79,18 @@ def run_def(L, seed, rs, difficulty=1, random_agent=True, max_steps=1200, multi=
         check_step(tag, env, o, obs, rew, done, out, out.reward, step)
         assert info["AllowNextMove"] == bool(out.allow_next_def)
         assert info["Win"] == (None if out.win < 0 else bool(out.win))
-        if done:
+        if _episode_over(done, left):
             break
     return step
 
 
-def run_atk(L, seed, rs, difficulty=1, max_steps=1200):
+def run_atk(L, seed, rs, difficulty=1, max_steps=1200, past_done=0):
     seed, env = RH.first_valid_seed("atk", L, seed, difficulty=difficulty, random_agent=True)
     o = oracle_from_ref_env(env, current_oracle_config())
     random.seed(seed)
     o.set_pyrand(random.getstate())
     tag = "atk L=%d seed=%d diff=%d" % (L, seed, difficulty)
+    left = [past_done, False]
     for step in range(1, max_steps + 1):
         mode = rs.randint(4)
         if mode == 0:
@@ -94,15 +108,16 @@ def run_atk(L, seed, rs, difficulty=1, max_steps=1200):
         assert list(info["FailCode"]) == list(out.fail_atk[:out.n_fail_atk]), (tag, step)
         assert info["AllowNextMove"] == bool(out.allow_next_atk)
         assert info["Win"] == (None if out.win < 0 else bool(out.win))
-        if done:
+        if _episode_over(done, left):
             break
     return step
 
 
-def run_multi(L, seed, rs, max_steps=1200, multi=False):
+def run_multi(L, seed, rs, max_steps=1200, multi=False, past_done=0):
     seed, env = RH.first_valid_seed("2p", L, seed)
     o = oracle_from_ref_env(env, current_oracle_config())
     tag = "2p L=%d seed=%d multi=%s" % (L, seed, multi)
+    left = [past_done, False]
     for step in range(1, max_steps + 1):
         atk = np.full((3, 8), 4, dtype=np.int64)
         if rs.randint(3) == 0:
@@ -133,6 +148,7 @@ def run_multi(L, seed, rs, max_steps=1200, multi=False):
                                          "Defender": bool(out.allow_next_def)}
         if done:
             assert info["Win"] == {"Defender": bool(out.win), "Attacker": bool(out.win_attacker)}
+        if _episode_over(done, left):
             break
     return step
 

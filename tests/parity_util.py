@@ -17,6 +17,25 @@ from oracle import td_oracle as TO
 
 
 LAST_MAX = {"towers": 0, "enemies": 0}      # longest lists seen by the last run_parity (coverage evidence)
+LAST_RUN = {}                                # what the last run_parity went through: post-done steps, overflows, episodes
+
+
+def enemy_capacity(L):
+    """Live enemies the step kernel holds: one per lane on 10x10 boards, 64 otherwise."""
+    return 32 if L == 10 else E.CAP_ENEMIES
+
+
+def stats_reduction_order(values):
+    """Sum per-env f64 values in the order of td_stats_kernel (256 strided partial sums, then a halving tree)."""
+    r = [0.0] * 256
+    for i, v in enumerate(values):
+        r[i % 256] += v
+    stride = 128
+    while stride:
+        for t in range(stride):
+            r[t] += r[t + stride]
+        stride >>= 1
+    return r[0]
 
 
 def oracle_config_from_engine(cfg):
@@ -144,19 +163,40 @@ def compare_state(tag, eng, rec, o):
 
 
 def run_parity(kind, L, n_envs, steps, seed=0, multi=False, opponent="device", difficulty=1, cfg_overrides=None,
-               check_state_every=1, device=0, use_host_api=False, multi_mode="sparse", incremental=False):
+               check_state_every=1, device=0, use_host_api=False, multi_mode="sparse", incremental=False,
+               past_done=0, overflow="forbid", generic_kernels=False, auto_reset=False):
     """Step `n_envs` instances on the GPU and in the oracle; compare everything each step.
 
     opponent: "device" (on-device CPython-compatible generator), "stream" (host-resolved type/road
     bytes, DEF only) or "none".  Returns the number of env-steps compared.
+
+    past_done: steps every env keeps taking after its episode ended (auto-reset is off, and the reference has no
+    done latch), with fresh actions, still compared with its oracle twin, which keeps stepping too.
+
+    overflow: "forbid" -- no env may overflow its tower / enemy capacity; "expect" -- the header flags are read
+    after every step, an env's overflow flag must rise on exactly the step where the oracle's tower list first
+    exceeds 32 or its enemy list first exceeds enemy_capacity(L) (at any point inside the step), and the env is
+    compared bit for bit until then and dropped from that step on.
+
+    auto_reset: the step kernel restarts a finished env on its map (map_stride = n_envs) inside the step; the oracle
+    twin is rebuilt on the same map and keeps its opponent stream.
+
+    The episode statistics of the handle (td_get_stats) are checked against the oracle run at the end: every
+    episode counts once, on the step where it ends.
     """
     import torch
+    assert overflow in ("forbid", "expect") and not (auto_reset and past_done)
     dev = torch.device("cuda", device)
     LAST_MAX.update(towers=0, enemies=0)
+    LAST_RUN.clear()
+    LAST_RUN.update(post_done_steps=0, overflows=0, episodes=0)
     rs = np.random.RandomState(seed)
     cfg = make_config(**(cfg_overrides or {}))
     ocfg = oracle_config_from_engine(cfg)
     eng = E.Engine(kind, L, n_envs, device=device, cfg=cfg)
+    if generic_kernels:
+        eng.set_option("generic_kernels", 1)
+    ecap = enemy_capacity(L)
     seeds = (np.arange(n_envs, dtype=np.uint32) * 7 + 1000 * seed + 11).astype(np.uint32)
     maps, seeds, _ = mapgen.generate_batch(seeds, L)
     eng.upload_maps(maps)
@@ -193,8 +233,12 @@ def run_parity(kind, L, n_envs, steps, seed=0, multi=False, opponent="device", d
     atk_act = torch.zeros((n_envs, 3, 8), dtype=torch.int64, device=dev)
     opp = torch.zeros(n_envs, dtype=torch.uint8, device=dev)
     alive = np.ones(n_envs, dtype=bool)
+    extra = np.full(n_envs, past_done, dtype=np.int64)       # steps still to take after done
+    ended = np.zeros(n_envs, dtype=bool)
+    overflowed = np.zeros(n_envs, dtype=bool)
+    episodes = [[] for _ in range(n_envs)]                   # (return, length, win, kills, leaks) per finished episode
+    ep_ret, ep_kills, ep_leaks = [0.0] * n_envs, [0] * n_envs, [0] * n_envs
     compared = 0
-    outs = [None] * n_envs
     for step in range(1, steps + 1):
         a_def = np.zeros(def_shape, dtype=np.int64)
         a_atk = np.full((n_envs, 3, 8), 4, dtype=np.int64)
@@ -218,7 +262,7 @@ def run_parity(kind, L, n_envs, steps, seed=0, multi=False, opponent="device", d
         io = E.Engine.make_io(def_action=def_act if kind != "atk" else None,
                               atk_action=atk_act if kind != "def" else None,
                               opponent=opp if (kind == "def" and opponent == "stream") else None,
-                              multi_action=multi, auto_reset=False, obs=obs, reward=t["reward"], done=t["done"],
+                              multi_action=multi, auto_reset=auto_reset, obs=obs, reward=t["reward"], done=t["done"],
                               win=t["win"], allow_next=t["allow_next"], real_def=t["real_def"],
                               real_atk=t["real_atk"], fail_def=t["fail_def"], fail_atk=t["fail_atk"],
                               obs_incremental=incremental)
@@ -227,11 +271,13 @@ def run_parity(kind, L, n_envs, steps, seed=0, multi=False, opponent="device", d
         torch.cuda.synchronize()
         host = {k: v.cpu().numpy() for k, v in t.items()}
         obs_h = obs.cpu().numpy()
-        recs = eng.get_state_raw() if (step % check_state_every == 0 or step == steps) else None
+        check_state = step % check_state_every == 0 or step == steps
+        recs = eng.get_state_raw() if (check_state or overflow == "expect") else None
         for i, o in enumerate(oracles):
             if not alive[i]:
                 continue
-            tag = "%s L=%d env=%d step=%d" % (kind, L, i, step)
+            tag = "%s L=%d env=%d step=%d%s" % (kind, L, i, step, " (after done)" if ended[i] else "")
+            o.e.peak_towers, o.e.peak_enemies = o.e.n_towers, o.e.n_enemies
             real_multi = None
             if kind == "def":
                 if multi:
@@ -250,6 +296,19 @@ def run_parity(kind, L, n_envs, steps, seed=0, multi=False, opponent="device", d
                     out, real_multi = o.multi_step_multi(a_atk[i], a_def[i])
                 else:
                     out = o.multi_step(a_atk[i], int(a_def[i]))
+            over = o.e.peak_towers > E.CAP_TOWERS or o.e.peak_enemies > ecap
+            if overflow == "expect":
+                flags = int(eng.decode_state(recs[i])["header"]["flags"])
+                assert flags & ~3 == 0, tag + " internal check failed (flags %#x)" % flags
+                assert bool(flags) == over, tag + " overflow flag %#x, oracle peak lists %d towers / %d enemies (cap %d / %d)" % (
+                    flags, o.e.peak_towers, o.e.peak_enemies, E.CAP_TOWERS, ecap)
+                if over:
+                    alive[i] = False                 # past its capacity the env is no longer the reference's
+                    overflowed[i] = True
+                    LAST_RUN["overflows"] += 1
+                    continue
+            assert not over, tag + " the oracle's lists exceed the capacity (%d towers, %d enemies): use overflow='expect'" % (
+                o.e.peak_towers, o.e.peak_enemies)
             assert float(host["reward"][i]).hex() == float(out.reward).hex(), \
                 "%s reward %r != %r" % (tag, host["reward"][i], out.reward)
             assert bool(host["done"][i]) == bool(out.done), tag + " done"
@@ -269,21 +328,59 @@ def run_parity(kind, L, n_envs, steps, seed=0, multi=False, opponent="device", d
                 want = [out.n_fail_atk] + list(out.fail_atk[:out.n_fail_atk])
                 got = host["fail_atk"][i].tolist()
                 assert got[:1 + out.n_fail_atk] == want, tag + " fail_atk %r != %r" % (got, want)
+            if not ended[i]:
+                ep_ret[i] += out.reward
+                ep_kills[i] += o.e.last_kills
+                ep_leaks[i] += o.e.last_leaks
+                if out.done:
+                    episodes[i].append((ep_ret[i], o.e.steps, int(out.win), ep_kills[i], ep_leaks[i]))
+                    if auto_reset:
+                        py = o.e.pyrand
+                        oracles[i] = o = oracle_env_from_map(maps[i], ocfg)
+                        o.e.pyrand = py
+                        ep_ret[i], ep_kills[i], ep_leaks[i] = 0.0, 0, 0
+                    else:
+                        ended[i] = True
+            elif not out.done:
+                raise AssertionError(tag + " a finished env must report done on every later step")
+            else:
+                LAST_RUN["post_done_steps"] += 1
             oo = o.get_states()
             if not np.array_equal(obs_h[i].view(np.uint32), oo.view(np.uint32)):
                 ch = sorted(set(np.argwhere(obs_h[i] != oo)[:, 0].tolist()))
                 raise AssertionError("%s obs differs in channels %s" % (tag, ch))
-            if recs is not None:
+            if check_state:
                 compare_state(tag, eng, recs[i], o)
             compared += 1
             LAST_MAX["towers"] = max(LAST_MAX["towers"], o.e.n_towers)
             LAST_MAX["enemies"] = max(LAST_MAX["enemies"], o.e.n_enemies)
-            if out.done:
-                alive[i] = False
+            if ended[i]:
+                if extra[i] == 0:
+                    alive[i] = False
+                extra[i] -= 1
         if not alive.any():
             break
     st = eng.stats()
-    assert st["overflow_envs"] == 0, "capacity overflow flagged"
+    if overflow == "forbid":
+        assert st["overflow_envs"] == 0, "capacity overflow flagged"
+    else:
+        assert st["overflow_envs"] == int(overflowed.sum()), "overflow flagged on %d envs, expected %d" % (
+            st["overflow_envs"], overflowed.sum())
+    # statistics: envs that overflowed go on with lists the reference does not have; leave them out
+    if not overflowed.any():
+        eps = [w for per_env in episodes for w in per_env]
+        LAST_RUN["episodes"] = len(eps)
+        got = (st["episodes"], st["length_sum"], st["wins"], st["kills"], st["leaks"])
+        want = (len(eps), sum(w[1] for w in eps), sum(w[2] for w in eps), sum(w[3] for w in eps), sum(w[4] for w in eps))
+        assert got == want, "stats (episodes, length, wins, kills, leaks) %r != %r" % (got, want)
+        per_env = []
+        for ep in episodes:                                  # EnvStats.return_sum: the env's episodes in order
+            r = 0.0
+            for w in ep:
+                r += w[0]
+            per_env.append(r)
+        want_ret = stats_reduction_order(per_env)
+        assert float(st["return_sum"]).hex() == float(want_ret).hex(), "stats return %r != %r" % (st["return_sum"], want_ret)
     eng.close()
     return compared
 
