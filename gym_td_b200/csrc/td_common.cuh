@@ -454,6 +454,8 @@ __device__ __forceinline__ void reset_env(W &w, const StepParams &p, int map_id,
         w.hdr()->ep_return = 0.0;
         w.hdr()->ep_kills = 0;
         w.hdr()->ep_leaks = 0;
+        w.hdr()->ep_kills_hi = 0;
+        w.hdr()->ep_leaks_hi = 0;
     }
     gsync(w);
 }

@@ -140,6 +140,12 @@ static int validate_config(td_handle *h, const td_config *c)
         for (int l = 0; l < TD_NLV; ++l)
             if (c->tower_range[t][l] < 0 || c->tower_splash_range[t][l] < 0 || !(c->enemy_LP[t][l] > 0))
                 return fail(h, TD_E_INVALID, "negative range or non-positive enemy LP in config tables");
+    // observation planes 11-12 divide by max_cost, 41-44 by enemy_cost[t][0]: the reference divides Python numbers
+    // there (TDBoard.py:118,123-125,142) and raises ZeroDivisionError, so it cannot run such a config (DESIGN.md 5)
+    if (!(c->max_cost > 0)) return fail(h, TD_E_INVALID, "max_cost must be > 0 (and not NaN)");
+    for (int t = 0; t < TD_NTYPES; ++t)
+        if (c->enemy_cost[t][0] == 0 || c->enemy_cost[t][0] != c->enemy_cost[t][0])
+            return fail(h, TD_E_INVALID, "enemy_cost[t][0] must not be 0 or NaN");
     return TD_OK;
 }
 
@@ -666,10 +672,13 @@ static int check_io(td_handle *h, const td_step_io *io)
 }
 
 // launch the fused step for envs [begin, begin + count) on `s`
-// td_step_io.obs_incremental is honoured only for the buffer the library itself filled last
+// td_step_io.obs_incremental is honoured only for the buffer the library itself filled last, and only when that buffer
+// is 16-byte aligned: the in-place update stores float4 (obs_dense_incremental); elsewhere the full write takes its
+// scalar path
 static bool obs_is_current(const td_handle *h, const td_step_io *io)
 {
-    return io->obs_incremental != 0 && io->obs_format == TD_OBS_F32 && io->obs_dev != nullptr && io->obs_dev == h->obs_synced;
+    return io->obs_incremental != 0 && io->obs_format == TD_OBS_F32 && io->obs_dev != nullptr && io->obs_dev == h->obs_synced &&
+           (reinterpret_cast<uintptr_t>(io->obs_dev) & 15) == 0;
 }
 
 // Where a step kernel goes: straight onto a stream, or into a graph under construction (td_step_host).
@@ -1175,18 +1184,28 @@ extern "C" int td_set_state(td_handle *h, int first_env, int n, const void *blob
     h->obs_synced = nullptr;                                    // no buffer shows the state being written
     if (!blob || first_env < 0 || n < 1 || first_env + n > h->n_envs) return fail(h, TD_E_INVALID, "td_set_state: bad range");
     const uint8_t *b = static_cast<const uint8_t *>(blob);
+    // the step kernels hold one enemy per lane on 10x10 boards (td_kernels.cuh: ecap = GW * NCHUNK = 32)
+    const int enemy_cap = h->L == 10 ? 32 : TD_CAP_ENEMIES;
     for (int i = 0; i < n; ++i) {
-        const td_env_header *hd = reinterpret_cast<const td_env_header *>(b + (size_t)i * h->record_bytes);
-        if (hd->n_towers > TD_CAP_TOWERS || hd->n_enemies > TD_CAP_ENEMIES || hd->map_id < 0 ||
+        const uint8_t *rec = b + (size_t)i * h->record_bytes;
+        const td_env_header *hd = reinterpret_cast<const td_env_header *>(rec);
+        if (hd->n_towers > TD_CAP_TOWERS || hd->n_enemies > enemy_cap || hd->map_id < 0 ||
             (h->n_maps > 0 && hd->map_id >= h->n_maps) || hd->rng_pos < 0 || hd->rng_pos > kMtWords ||
             hd->pad0 > h->rng_cache_words || hd->pad1 < 0 || hd->pad1 > hd->pad0)
             return fail(h, TD_E_INVALID, "td_set_state: record header out of range");
-        const td_tower_rec *tw = reinterpret_cast<const td_tower_rec *>(b + (size_t)i * h->record_bytes + h->off_towers);
+        // road bits of the record's own static map: enemies walk the road (movement follows its direction bits and
+        // would leave the board from any other cell, or from the end cell, where the reference removes them), towers
+        // stand beside it
+        const MapHdr *mh = reinterpret_cast<const MapHdr *>(rec + h->off_static);
+        const uint8_t *road = rec + h->off_static + kMapHdrBytes;
+        const td_tower_rec *tw = reinterpret_cast<const td_tower_rec *>(rec + h->off_towers);
         for (int t = 0; t < hd->n_towers; ++t)
-            if (tw[t].loc >= h->cells || (tw[t].type_lv >> 2) >= TD_NLV) return fail(h, TD_E_INVALID, "td_set_state: bad tower record");
-        const td_enemy_rec *en = reinterpret_cast<const td_enemy_rec *>(b + (size_t)i * h->record_bytes + h->off_enemies);
+            if (tw[t].loc >= h->cells || (tw[t].type_lv >> 2) >= TD_NLV || (road[tw[t].loc] & 1))
+                return fail(h, TD_E_INVALID, "td_set_state: bad tower record");
+        const td_enemy_rec *en = reinterpret_cast<const td_enemy_rec *>(rec + h->off_enemies);
         for (int e = 0; e < hd->n_enemies; ++e)
-            if (en[e].loc >= h->cells || (en[e].type_lv >> 2) >= TD_NLV) return fail(h, TD_E_INVALID, "td_set_state: bad enemy record");
+            if (en[e].loc >= h->cells || (en[e].type_lv >> 2) >= TD_NLV || !(road[en[e].loc] & 1) || en[e].loc == mh->end)
+                return fail(h, TD_E_INVALID, "td_set_state: bad enemy record");
     }
     TD_CUDA(h, cudaSetDevice(h->device));
     TD_CUDA(h, cudaDeviceSynchronize());

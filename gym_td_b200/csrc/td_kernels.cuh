@@ -216,8 +216,13 @@ __device__ __forceinline__ void env_rules(const StepParams &p, const int env, W 
         }
         td_env_header *h = w.hdr();
         h->ep_return = __dadd_rn(h->ep_return, reward);
-        h->ep_kills = (uint16_t)(h->ep_kills + kills);
-        h->ep_leaks = (uint16_t)(h->ep_leaks + leaks);
+        // 32-bit episode counters kept as two 16-bit halves of the header
+        const uint32_t ep_kills = ((uint32_t)h->ep_kills | ((uint32_t)h->ep_kills_hi << 16)) + (uint32_t)kills;
+        const uint32_t ep_leaks = ((uint32_t)h->ep_leaks | ((uint32_t)h->ep_leaks_hi << 16)) + (uint32_t)leaks;
+        h->ep_kills = (uint16_t)ep_kills;
+        h->ep_kills_hi = (uint16_t)(ep_kills >> 16);
+        h->ep_leaks = (uint16_t)ep_leaks;
+        h->ep_leaks_hi = (uint16_t)(ep_leaks >> 16);
         // An episode counts once, on the step where it ends.  A finished env that is stepped on without a reset
         // (auto_reset off; the reference has no done latch) reports done again: the header in the slice still holds
         // the pre-step base_LP / steps, and an env that had already ended before this step is not counted again.
@@ -228,8 +233,8 @@ __device__ __forceinline__ void env_rules(const StepParams &p, const int env, W 
             s.episodes += 1;
             s.wins += my_win ? 1 : 0;
             s.length_sum += (uint32_t)w.steps;
-            s.kills += h->ep_kills;
-            s.leaks += h->ep_leaks;
+            s.kills += ep_kills;
+            s.leaks += ep_leaks;
         }
         if (w.flags) p.stats[env].flags |= (uint32_t)w.flags;
     }

@@ -75,7 +75,7 @@ HEADER_DTYPE = np.dtype([
     ("cost_def", "<f8"), ("cost_atk", "<f8"), ("ep_return", "<f8"), ("base_LP", "<i4"), ("steps", "<i4"),
     ("map_id", "<i4"), ("episode", "<i4"), ("defender_cd", "<i2"), ("attacker_cd", "<i2"),
     ("n_towers", "u1"), ("n_enemies", "u1"), ("flags", "u1"), ("pad0", "u1"), ("ep_kills", "<u2"),
-    ("ep_leaks", "<u2"), ("rng_pos", "<i4"), ("pad1", "<i4"), ("pad2", "<i4")])
+    ("ep_leaks", "<u2"), ("rng_pos", "<i4"), ("pad1", "<i4"), ("ep_kills_hi", "<u2"), ("ep_leaks_hi", "<u2")])
 TOWER_DTYPE = np.dtype([("cd", "<f8"), ("loc", "<u2"), ("type_lv", "u1"), ("scratch", "u1", (5,))])
 ENEMY_DTYPE = np.dtype([("LP", "<f8"), ("margin", "<f8"), ("loc", "<u2"), ("type_lv", "u1"),
                         ("slowdown", "u1"), ("scratch", "u1", (4,))])
@@ -217,6 +217,11 @@ def config_struct(cfg=None, hyper=None):
             setattr(c, name, d[name])
     if "base_LP" in d:
         c.base_LP = _base_lp(d["base_LP"])
+    # the observation divides by these (TDBoard.py:118,123-125,142); the reference raises ZeroDivisionError there
+    if not c.max_cost > 0:
+        raise ValueError("max_cost must be > 0 (and not NaN), got %r" % (c.max_cost,))
+    if any(c.enemy_cost[t][0] == 0 or c.enemy_cost[t][0] != c.enemy_cost[t][0] for t in range(NT)):
+        raise ValueError("enemy_cost[t][0] must not be 0 or NaN, got %r" % ([c.enemy_cost[t][0] for t in range(NT)],))
     c.max_episode_steps = int(hyper.get("max_episode_steps", 1200))
     return c
 

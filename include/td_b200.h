@@ -43,7 +43,8 @@ extern "C" {
 #define TD_ABI_VERSION 3   /* 2: td_step_io grew `obs_incremental` (+ reserved_) at its end; 3: td_set_option,
                               config per handle, td_step_host as one graph launch.  Added since, without a layout
                               change: TD_OPT_GENERIC_KERNELS / HOST_CHAIN / HOST_FIRST_CHUNK / HOST_ZERO_COPY,
-                              td_alloc_compressible / td_free_compressible */
+                              td_alloc_compressible / td_free_compressible, td_env_header.ep_kills_hi / ep_leaks_hi
+                              in the formerly unused pad2 word */
 
 enum { TD_OK = 0, TD_E_INVALID = -1, TD_E_CUDA = -2, TD_E_ALLOC = -3, TD_E_STATE = -4,
        TD_E_OVERFLOW = -5 };
@@ -141,7 +142,7 @@ typedef struct td_step_io {
                                         tensor is bit-identical to a full write.  Ignored (full write) whenever the
                                         library cannot vouch for the buffer: another pointer than last time, after
                                         td_set_state, for envs that were reset inside the step, for board sizes
-                                        without a specialised kernel. */
+                                        without a specialised kernel, for a buffer that is not 16-byte aligned. */
     int32_t obs_format;              /* TD_OBS_F32 (0, default): obs_dev is float32, the reference layout.  TD_OBS_BF16 /
                                         TD_OBS_U8 (ABI 3): obs_dev points to [n,45,L,L] bfloat16 / uint8 elements instead
                                         (SURVEY 8(f) f4, reduced-precision planes): bf16 = the float32 value rounded to
@@ -201,11 +202,12 @@ typedef struct td_env_header {
     uint8_t n_enemies;
     uint8_t flags;              /* bit0 enemy overflow, bit1 tower overflow (sticky) */
     uint8_t pad0;               /* internal: valid words of the record's generator word cache */
-    uint16_t ep_kills;
+    uint16_t ep_kills;          /* kills / leaks of the running episode: low 16 bits ... */
     uint16_t ep_leaks;
     int32_t rng_pos;            /* position in the opponent MT19937 state (0..624) */
     int32_t pad1;               /* internal: consumed words of that cache */
-    int32_t pad2;
+    uint16_t ep_kills_hi;       /* ... and high 16 bits (an episode may last INT_MAX steps; this word was pad2) */
+    uint16_t ep_leaks_hi;
 } td_env_header;                /* 64 bytes */
 
 typedef struct td_tower_rec {   /* 16 bytes, list order */

@@ -382,6 +382,36 @@ static void enemy_damage(tdo_enemy *en, double atk, int magic)
     en->hit = 1;
 }
 
+/* TDBoard.py:355-365: enemy statistics of the current lists, float32 in list order (NumPy 2 / NEP 50 semantics).
+ * The last part of tdo_board_step; also callable on its own for a state written field by field. */
+void tdo_enemy_stats(tdo_env *e)
+{
+    const int cells = e->L * e->L;
+    for (int t = 0; t < TDO_NTYPES; ++t)
+        for (int c = 0; c < cells; ++c) {
+            e->enemy_LP[0][t][c] = 1.f;
+            e->enemy_LP[1][t][c] = 0.f;
+            e->enemy_LP[2][t][c] = 0.f;
+            e->enemy_LP[3][t][c] = 0.f;
+        }
+    for (int i = 0; i < e->n_enemies; ++i) {
+        const tdo_enemy *en = &e->enemies[i];
+        float r = (float)(en->LP / en->maxLP);
+        float *mn = &e->enemy_LP[0][en->type][en->loc], *mx = &e->enemy_LP[1][en->type][en->loc];
+        if (r < *mn) *mn = r;
+        if (r > *mx) *mx = r;
+        e->enemy_LP[2][en->type][en->loc] += r;
+        e->enemy_LP[3][en->type][en->loc] += 1.f;
+    }
+    for (int t = 0; t < TDO_NTYPES; ++t)
+        for (int c = 0; c < cells; ++c) {
+            float cnt = e->enemy_LP[3][t][c];
+            if (!(cnt > 0)) { e->enemy_LP[0][t][c] = 0.f; e->enemy_LP[2][t][c] = 0.f; }
+            else e->enemy_LP[2][t][c] = e->enemy_LP[2][t][c] / cnt;
+            e->enemy_LP[3][t][c] = cnt / (float)TDO_CLUSTER;
+        }
+}
+
 /* TDBoard.py:295-368 */
 double tdo_board_step(tdo_env *e)
 {
@@ -485,31 +515,7 @@ double tdo_board_step(tdo_env *e)
     double cd = e->cost_def + e->cfg.defender_cost_rate;
     e->cost_def = e->max_cost < cd ? e->max_cost : cd;
 
-    /* :355-365 enemy statistics, float32 in list order (NumPy 2 / NEP 50 semantics) */
-    const int cells = L * L;
-    for (int t = 0; t < TDO_NTYPES; ++t)
-        for (int c = 0; c < cells; ++c) {
-            e->enemy_LP[0][t][c] = 1.f;
-            e->enemy_LP[1][t][c] = 0.f;
-            e->enemy_LP[2][t][c] = 0.f;
-            e->enemy_LP[3][t][c] = 0.f;
-        }
-    for (int i = 0; i < e->n_enemies; ++i) {
-        const tdo_enemy *en = &e->enemies[i];
-        float r = (float)(en->LP / en->maxLP);
-        float *mn = &e->enemy_LP[0][en->type][en->loc], *mx = &e->enemy_LP[1][en->type][en->loc];
-        if (r < *mn) *mn = r;
-        if (r > *mx) *mx = r;
-        e->enemy_LP[2][en->type][en->loc] += r;
-        e->enemy_LP[3][en->type][en->loc] += 1.f;
-    }
-    for (int t = 0; t < TDO_NTYPES; ++t)
-        for (int c = 0; c < cells; ++c) {
-            float cnt = e->enemy_LP[3][t][c];
-            if (!(cnt > 0)) { e->enemy_LP[0][t][c] = 0.f; e->enemy_LP[2][t][c] = 0.f; }
-            else e->enemy_LP[2][t][c] = e->enemy_LP[2][t][c] / cnt;
-            e->enemy_LP[3][t][c] = cnt / (float)TDO_CLUSTER;
-        }
+    tdo_enemy_stats(e);
     return reward;
 }
 

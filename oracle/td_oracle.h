@@ -144,6 +144,7 @@ int tdo_tower_destruct(tdo_env *e, int loc);
 int tdo_summon_enemy(tdo_env *e, int t, int start_id);
 int tdo_summon_cluster(tdo_env *e, const int64_t *types, int start_id, int64_t *real_act);
 double tdo_board_step(tdo_env *e);
+void tdo_enemy_stats(tdo_env *e);   /* the enemy-statistics planes of the current lists (end of tdo_board_step) */
 int tdo_done(const tdo_env *e);
 void tdo_get_states(const tdo_env *e, float *out);
 int tdo_n_channels(void);

@@ -224,6 +224,12 @@ class OracleEnv(object):
     def done(self):
         return bool(self.L_.tdo_done(C.byref(self.e)))
 
+    def refresh(self):
+        """Bring the derived fields in line with a state written field by field: progress (steps / max_episode_steps
+        in f64, as tdo_board_step computes it) and the enemy-statistics planes of the current lists (tdo_enemy_stats)."""
+        self.e.progress = float(self.e.steps) / float(self.e.cfg.max_episode_steps)
+        self.L_.tdo_enemy_stats(C.byref(self.e))
+
     def get_states(self):
         L = self.e.L
         out = np.empty((45, L, L), dtype=np.float32)

@@ -162,9 +162,108 @@ def compare_state(tag, eng, rec, o):
         raise AssertionError("%s: state mismatch: %s" % (tag, "; ".join(bad[:6])))
 
 
+# ------------------------------------------------------------------------------------------------
+# Constructed states: a board reached through the oracle's own API, then written into a CUDA env record
+
+BIG_PURSE = float("inf")          # no cost check fails while the lists are built
+
+
+def road_cells(o):
+    """Road cells of the oracle env other than the end cell, where an enemy can stand (r-major order)."""
+    e = o.e
+    cells = e.L * e.L
+    road = np.ctypeslib.as_array(e.road)[:cells] & 1
+    return [c for c in np.flatnonzero(road).tolist() if c != e.end]
+
+
+def free_cells(o):
+    """Cells where a tower can be built now (map6 == 0, r-major order)."""
+    e = o.e
+    return np.flatnonzero(np.ctypeslib.as_array(e.map6)[:e.L * e.L] == 0).tolist()
+
+
+def construct_state(o, towers=(), enemies=(), **header):
+    """Bring oracle env `o` (fresh from oracle_env_from_map) to a constructed state.
+
+    towers: (type, lv, loc, cd) in list order; tower_build, then tower_lvup for level 1, so the upgraded tower keeps
+    the reference's swapped constants (TDElements.py:163-169) and map6 its diamond counts; then cd is written.
+    cd None keeps the fresh tower's 0.
+    enemies: (type, lv, loc, margin, LP, slowdown) in list order; summon_enemy at the level `progress` selects,
+    then loc (a road cell, dist = dist[loc]), margin in [0, 1), LP in (0, maxLP] (None: maxLP) and slowdown written.
+    header: cost_def, cost_atk, steps, defender_cd, attacker_cd, base_LP -- written last.
+    Purses are large while the lists are built.  Ends with refresh() (progress, enemy statistics).  The enemies'
+    levels, which the oracle does not store, are kept in o.enemy_lv (list order)."""
+    e = o.e
+    cells = e.L * e.L
+    road = np.ctypeslib.as_array(e.road)[:cells] & 1
+    for t, lv, loc, cd in towers:
+        assert not road[loc], "tower on a road cell"
+        e.cost_def = BIG_PURSE
+        assert o.tower_build(t, loc), "tower_build(%d, %d) failed (fail code %d)" % (t, loc, e.fail_code)
+        if lv:
+            assert o.tower_lvup(loc)
+        if cd is not None:
+            e.towers[e.n_towers - 1].cd = cd
+    levels = []
+    upgrade_at = e.cfg.enemy_upgrade_at
+    for t, lv, loc, margin, LP, slowdown in enemies:
+        assert road[loc] and loc != e.end, "enemy off the road"
+        assert 0.0 <= margin < 1.0 and 0 <= slowdown <= 255
+        e.cost_atk = BIG_PURSE
+        e.progress = 1e300 if lv else -1e300
+        assert (e.progress >= upgrade_at) == bool(lv), "enemy_upgrade_at %r leaves no level-%d summon" % (upgrade_at, lv)
+        assert o.summon_enemy(t, 0)
+        x = e.enemies[e.n_enemies - 1]
+        x.loc, x.dist, x.margin, x.slowdown = loc, e.dist[loc], margin, slowdown
+        if LP is not None:
+            assert 0.0 < LP <= x.maxLP, "LP %r outside (0, maxLP]" % (LP,)
+            x.LP = LP
+        levels.append(int(lv))
+    h = dict(cost_def=e.cfg.defender_init_cost, cost_atk=e.cfg.attacker_init_cost)
+    h.update(header)
+    for k, v in h.items():
+        if k == "base_LP":
+            assert e.has_base_LP, "base_LP of a config without a base"
+        setattr(e, k, v)
+    o.enemy_lv = levels
+    o.refresh()
+    return o
+
+
+def encode_record(eng, row, o, ep=None):
+    """Write oracle env `o` into the CUDA env record `row` (a row of eng.get_state_raw() of the same env, which keeps
+    its static map, generator word cache and rng_pos): the inverse of compare_state.  Enemy levels come from
+    o.enemy_lv (construct_state).  ep: optional (ep_return, ep_kills, ep_leaks) of the running episode."""
+    e, lay = o.e, eng.layout
+    cells = e.L * e.L
+    assert e.n_towers <= E.CAP_TOWERS and e.n_enemies <= E.CAP_ENEMIES
+    h = row[:64].view(E.HEADER_DTYPE)
+    h["cost_def"], h["cost_atk"] = e.cost_def, e.cost_atk
+    h["base_LP"] = e.base_LP if e.has_base_LP else -1
+    h["steps"], h["defender_cd"], h["attacker_cd"] = e.steps, e.defender_cd, e.attacker_cd
+    h["n_towers"], h["n_enemies"] = e.n_towers, e.n_enemies
+    if ep is not None:
+        h["ep_return"] = ep[0]
+        h["ep_kills"], h["ep_kills_hi"] = ep[1] & 0xffff, ep[1] >> 16
+        h["ep_leaks"], h["ep_leaks_hi"] = ep[2] & 0xffff, ep[2] >> 16
+    tw = row[lay.off_towers:lay.off_towers + 16 * E.CAP_TOWERS].view(E.TOWER_DTYPE)
+    for i in range(e.n_towers):
+        t = e.towers[i]
+        tw[i]["cd"], tw[i]["loc"], tw[i]["type_lv"] = t.cd, t.loc, t.type | (t.lv << 2)
+    en = row[lay.off_enemies:lay.off_enemies + 24 * E.CAP_ENEMIES].view(E.ENEMY_DTYPE)
+    assert len(o.enemy_lv) == e.n_enemies
+    for i in range(e.n_enemies):
+        x = e.enemies[i]
+        en[i]["LP"], en[i]["margin"], en[i]["loc"] = x.LP, x.margin, x.loc
+        en[i]["type_lv"], en[i]["slowdown"] = x.type | (o.enemy_lv[i] << 2), x.slowdown
+    row[lay.off_map6:lay.off_map6 + cells] = np.ctypeslib.as_array(e.map6)[:cells].astype(np.uint8)
+    return row
+
+
 def run_parity(kind, L, n_envs, steps, seed=0, multi=False, opponent="device", difficulty=1, cfg_overrides=None,
                check_state_every=1, device=0, use_host_api=False, multi_mode="sparse", incremental=False,
-               past_done=0, overflow="forbid", generic_kernels=False, auto_reset=False):
+               past_done=0, overflow="forbid", generic_kernels=False, auto_reset=False, prepare=None, inspect=None,
+               obs_offset=0, atk_policy=None):
     """Step `n_envs` instances on the GPU and in the oracle; compare everything each step.
 
     opponent: "device" (on-device CPython-compatible generator), "stream" (host-resolved type/road
@@ -183,13 +282,23 @@ def run_parity(kind, L, n_envs, steps, seed=0, multi=False, opponent="device", d
 
     The episode statistics of the handle (td_get_stats) are checked against the oracle run at the end: every
     episode counts once, on the step where it ends.
+
+    prepare: fn(i, oracle, rs) called for every env after the reset; it brings oracle env i to a constructed state
+    (construct_state) and may return (ep_return, ep_kills, ep_leaks) of the running episode.  Every env is then
+    written into its CUDA record (encode_record, td_set_state), td_observe must match get_states() bit for bit, and
+    the steps start from there.  inspect: fn(eng, oracles) called right after that check, before the first step.
+
+    obs_offset: the observation buffer starts this many float32 elements after a 256-byte aligned allocation
+    (1: 4 bytes off the 16-byte boundary, the scalar store path).
+
+    atk_policy: fn(rs) -> (3, 8) attacker action, in place of attacker_action.
     """
     import torch
     assert overflow in ("forbid", "expect") and not (auto_reset and past_done)
     dev = torch.device("cuda", device)
     LAST_MAX.update(towers=0, enemies=0)
     LAST_RUN.clear()
-    LAST_RUN.update(post_done_steps=0, overflows=0, episodes=0)
+    LAST_RUN.update(post_done_steps=0, overflows=0, episodes=0, max_ep_kills=0, max_ep_leaks=0)
     rs = np.random.RandomState(seed)
     cfg = make_config(**(cfg_overrides or {}))
     ocfg = oracle_config_from_engine(cfg)
@@ -211,12 +320,32 @@ def run_parity(kind, L, n_envs, steps, seed=0, multi=False, opponent="device", d
         eng.seed_opponent(states)
         eng.set_difficulty(difficulty)
 
-    obs = torch.empty((n_envs, 45, L, L), dtype=torch.float32, device=dev)
+    obs_buf = torch.empty(n_envs * 45 * cells + obs_offset, dtype=torch.float32, device=dev)
+    obs = obs_buf[obs_offset:].view(n_envs, 45, L, L)
     eng.reset(obs=obs)
     torch.cuda.synchronize()
     obs_h = obs.cpu().numpy()
     for i, o in enumerate(oracles):
         assert np.array_equal(obs_h[i].view(np.uint32), o.get_states().view(np.uint32)), "obs0 env %d" % i
+    ep0 = [(0.0, 0, 0)] * n_envs
+    if prepare is not None:
+        recs = eng.get_state_raw()
+        for i, o in enumerate(oracles):
+            ep0[i] = prepare(i, o, rs) or ep0[i]
+            encode_record(eng, recs[i], o, ep0[i])
+        eng.set_state_raw(recs)
+        eng.observe(obs)
+        torch.cuda.synchronize()
+        obs_h = obs.cpu().numpy()
+        for i, o in enumerate(oracles):
+            oo = o.get_states()
+            if not np.array_equal(obs_h[i].view(np.uint32), oo.view(np.uint32)):
+                ch = sorted(set(np.argwhere(obs_h[i].view(np.uint32) != oo.view(np.uint32))[:, 0].tolist()))
+                raise AssertionError("%s L=%d env=%d constructed state: td_observe differs in channels %s" % (kind, L, i, ch))
+            compare_state("%s L=%d env=%d constructed state" % (kind, L, i), eng, eng.get_state_raw(i, 1)[0], o)
+        if inspect is not None:
+            inspect(eng, oracles)
+            eng.observe(obs)                     # the step's in-place update trusts the buffer written last
 
     t = dict(
         reward=torch.zeros(n_envs, dtype=torch.float64, device=dev),
@@ -237,7 +366,7 @@ def run_parity(kind, L, n_envs, steps, seed=0, multi=False, opponent="device", d
     ended = np.zeros(n_envs, dtype=bool)
     overflowed = np.zeros(n_envs, dtype=bool)
     episodes = [[] for _ in range(n_envs)]                   # (return, length, win, kills, leaks) per finished episode
-    ep_ret, ep_kills, ep_leaks = [0.0] * n_envs, [0] * n_envs, [0] * n_envs
+    ep_ret, ep_kills, ep_leaks = [list(v) for v in zip(*ep0)]
     compared = 0
     for step in range(1, steps + 1):
         a_def = np.zeros(def_shape, dtype=np.int64)
@@ -252,7 +381,7 @@ def run_parity(kind, L, n_envs, steps, seed=0, multi=False, opponent="device", d
                 a_def[i] = ((uniform_multi_action(L, rs) if multi_mode == "uniform" else sparse_multi_action(L, rs))
                             if multi else smart_defender_action(o, rs))
             if kind != "def":
-                a_atk[i] = attacker_action(rs)
+                a_atk[i] = (atk_policy or attacker_action)(rs)
             if kind == "def" and opponent == "stream":
                 tt, rd = rs.randint(4), rs.randint(o.e.num_roads)
                 a_opp[i] = tt | (rd << 4)
@@ -332,6 +461,8 @@ def run_parity(kind, L, n_envs, steps, seed=0, multi=False, opponent="device", d
                 ep_ret[i] += out.reward
                 ep_kills[i] += o.e.last_kills
                 ep_leaks[i] += o.e.last_leaks
+                LAST_RUN["max_ep_kills"] = max(LAST_RUN["max_ep_kills"], ep_kills[i])
+                LAST_RUN["max_ep_leaks"] = max(LAST_RUN["max_ep_leaks"], ep_leaks[i])
                 if out.done:
                     episodes[i].append((ep_ret[i], o.e.steps, int(out.win), ep_kills[i], ep_leaks[i]))
                     if auto_reset:

@@ -84,6 +84,22 @@ def test_default_config_equals_reference_values():
         E.config_struct(cfg)
 
 
+@pytest.mark.parametrize("key,value", [("max_cost", 0), ("max_cost", -1.5), ("max_cost", float("nan")),
+                                       ("enemy_cost", [[8, 8], [0, 15], [40, 40], [30, 30]]),
+                                       ("enemy_cost", [[float("nan"), 8], [15, 15], [40, 40], [30, 30]])])
+def test_config_with_a_zero_divisor_is_rejected(key, value):
+    """Observation planes 11-12 divide by max_cost, 41-44 by enemy_cost[t][0]; the reference raises
+    ZeroDivisionError on such a config, the engine refuses it up front."""
+    cfg = params.Config()
+    setattr(cfg, key, value)
+    with pytest.raises(ValueError):
+        E.config_struct(cfg)
+    cfg = params.Config()
+    cfg.enemy_cost = [[8, 0], [15, 0], [40, 0], [30, 0]]            # level 1 never divides
+    cfg.max_cost = 1e-300
+    assert E.config_struct(cfg).max_cost == 1e-300
+
+
 def test_create_validates_and_reports():
     lib = E.lib()
     h = C.c_void_p()
