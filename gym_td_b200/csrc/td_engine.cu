@@ -22,37 +22,36 @@ using namespace td;
 struct HostCopy { void *dst; const void *src; size_t bytes; };     // one copy of td_step_host (either direction)
 
 struct td_handle {
-    int device, kind, L, cells, cells_pad, n_envs;
-    int n_maps, map_stride, difficulty;
-    int record_bytes, map_bytes, smem_per_warp, scratch_off;
-    int old_lists_off, act_stage_off;
-    const float *obs_synced;       // buffer that holds the current observation of every env (NULL: none known)
-    int off_static, off_towers, off_enemies, off_map6, rng_cache_words;
-    uint8_t *records;
-    uint8_t *maps;
-    uint32_t *mt;
-    EnvStats *stats;
-    td_stats *stats_dev;
-    bool opponent_seeded;
-    long long steps;
+    int device = 0, kind = 0, L = 0, cells = 0, cells_pad = 0, n_envs = 0;
+    int n_maps = 0, map_stride = 0, difficulty = 1;
+    int record_bytes = 0, map_bytes = 0, smem_per_warp = 0, scratch_off = 0;
+    int old_lists_off = 0, act_stage_off = 0;
+    const float *obs_synced = nullptr;   // buffer that holds the current observation of every env (NULL: none known)
+    int off_static = 0, off_towers = 0, off_enemies = 0, off_map6 = 0, rng_cache_words = 0;
+    uint8_t *records = nullptr;
+    uint8_t *maps = nullptr;
+    uint32_t *mt = nullptr;
+    EnvStats *stats = nullptr;
+    td_stats *stats_dev = nullptr;
+    bool opponent_seeded = false;
+    long long steps = 0;
     // td_step_host: the whole host-buffer step (action copies, chunk kernels, output copies) is one CUDA graph,
     // cached per distinct set of buffers
     struct HostGraph { std::vector<unsigned char> key; cudaGraphExec_t exec; unsigned long long used; };
     std::vector<HostGraph> host_graphs;
-    unsigned long long host_graph_clock;
-    cudaStream_t host_stream;      // stands in for the legacy default stream, which cannot launch graphs
-    int host_chunks;               // 0 = automatic
-    int host_graph;                // 1 = graph launch (default), 0 = plain stream launches
-    int step_smem_kb, obs_smem_kb; // experiments (td_set_option): lower the residency of the step / observe kernels
-    bool generic_kernels;          // td_set_option: never pick the opponent-specialised step kernels
-    bool host_chain;               // td_step_host graph: chunk kernels chained, or independent branches (default)
-    int host_first_chunk;          // td_step_host: envs in the first chunk (chunks grow x3); 0 = equal chunks, -1 = automatic
-    unsigned long long cfg_generation;
+    unsigned long long host_graph_clock = 0;
+    cudaStream_t host_stream = nullptr;  // stands in for the legacy default stream, which cannot launch graphs
+    int host_chunks = 0;                 // 0 = automatic
+    int host_graph = 1;                  // 1 = graph launch (default), 0 = plain stream launches
+    bool generic_kernels = false;        // td_set_option: never pick the opponent-specialised step kernels
+    bool host_chain = false;             // td_step_host graph: chunk kernels chained, or independent branches (default)
+    int host_first_chunk = -1;           // td_step_host: envs in the first chunk (chunks grow x3); 0 = equal chunks, -1 = automatic
+    unsigned long long cfg_generation = 0;
     std::vector<unsigned char> host_key;   // td_step_host: lookup key of the call in progress
     std::vector<HostCopy> host_in, host_out;   // td_step_host: copy lists of the call in progress
-    int host_zero_copy;            // td_step_host inputs read by the kernel from host memory: -1 automatic (8-byte actions), 0 never, 1 always
-    td_config cfg;
-    DevConfig dev_cfg;             // derived tables of cfg; copied into the parameters of every launch (per handle)
+    int host_zero_copy = -1;             // td_step_host inputs read by the kernel from host memory: -1 automatic (8-byte actions), 0 never, 1 always
+    td_config cfg = {};
+    DevConfig dev_cfg = {};              // derived tables of cfg; copied into the parameters of every launch (per handle)
     std::string err;
 };
 
@@ -252,8 +251,6 @@ static void fill_params(const td_handle *h, StepParams &p)
 static int grid_of(const td_handle *h) { return (h->n_envs + kWarpsPerCta - 1) / kWarpsPerCta; }
 static size_t smem_of(const td_handle *h) { return (size_t)kWarpsPerCta * h->smem_per_warp; }
 
-// The step kernel is specialised on (env kind, multi-action) x (board size, enemy chunks): 10x10 boards hold at
-// most 32 live enemies (one per lane), larger boards 64; other sizes take the run-time-size variant.
 #ifndef TD_GROUP_SMALL
 #define TD_GROUP_SMALL 32     // lanes per game instance on 10x10 boards.  16 (two instances per warp) is
                               // correct and makes the rules 10 % faster, but the full step 6 % slower on B200:
@@ -281,15 +278,11 @@ static size_t step_smem_bytes(const td_handle *h)
 static int step_warps_per_cta(const td_handle *h, bool incremental)
 {
     // (10x10 boards only: at 20x20 it changes nothing, 0.1921 vs 0.1916 ms)
-#ifdef TD_ATK_WARPS_PER_CTA       // experiment: CTA size of the full-write attacker kernel on 10x10 boards (1 / 2 / 4 warps:
-                                  // 0.2369 / 0.2384 / 0.2390 ms before the OPP specialisation, 0.2293 vs 0.2287 ms after it)
-    if (!incremental && h->kind == TD_KIND_ATK && h->L == 10 && step_group_width(h) == 32) return TD_ATK_WARPS_PER_CTA;
-#endif
     return incremental && h->L == 10 && step_group_width(h) == 32 ? 1 : kWarpsPerCta;
 }
 
 // The scripted opponent of level 1 draws from the device generator and no host-resolved opponent input is set:
-// the case the specialised kernels (variants 5-7, OPP = 1) are compiled for.
+// the case the opponent-specialised kernels (OPP = 1) are compiled for.
 static bool scripted_lv1_on_device(const td_handle *h, const td_step_io *io)
 {
     return !h->generic_kernels && h->kind != TD_KIND_2P && h->difficulty == 1 && h->opponent_seeded && h->mt != nullptr &&
@@ -297,56 +290,86 @@ static bool scripted_lv1_on_device(const td_handle *h, const td_step_io *io)
            (h->kind != TD_KIND_ATK || io->def_action_dev == nullptr);
 }
 
-static int step_variant(const td_handle *h, const td_step_io *io)
-{
-    const bool multi = io->multi_action != 0;
-    if (scripted_lv1_on_device(h, io)) return h->kind == TD_KIND_DEF ? (multi ? 6 : 5) : 7;
-    return h->kind == TD_KIND_DEF ? (multi ? 1 : 0) : h->kind == TD_KIND_ATK ? 2 : (multi ? 4 : 3);
-}
+using StepKernel = void (*)(StepParams);
 
-template <int CELLS, int NCHUNK, int GW, bool INC, typename F> static cudaError_t for_each_kind(F f)
+// float32 observation kernels of one board specialisation.  `scripted`: the default scripted opponent (level 1 on
+// the device generator) known at compile time, for the defender and the attacker env.
+template <int CELLS, int NCHUNK, int GW, bool INC> static StepKernel f32_step_kernel(int kind, bool multi, bool scripted)
 {
-    cudaError_t e;
-    if ((e = f(td_step_kernel<TD_KIND_DEF, false, CELLS, NCHUNK, GW, INC>)) != cudaSuccess) return e;
-    if ((e = f(td_step_kernel<TD_KIND_DEF, true, CELLS, NCHUNK, GW, INC>)) != cudaSuccess) return e;
-    if ((e = f(td_step_kernel<TD_KIND_ATK, false, CELLS, NCHUNK, GW, INC>)) != cudaSuccess) return e;
-    if ((e = f(td_step_kernel<TD_KIND_2P, false, CELLS, NCHUNK, GW, INC>)) != cudaSuccess) return e;
-    if ((e = f(td_step_kernel<TD_KIND_2P, true, CELLS, NCHUNK, GW, INC>)) != cudaSuccess) return e;
-    // variants 5-7: the default scripted opponent (level 1 on the device generator) known at compile time
-    if ((e = f(td_step_kernel<TD_KIND_DEF, false, CELLS, NCHUNK, GW, INC, float, 1>)) != cudaSuccess) return e;
-    if ((e = f(td_step_kernel<TD_KIND_DEF, true, CELLS, NCHUNK, GW, INC, float, 1>)) != cudaSuccess) return e;
-    return f(td_step_kernel<TD_KIND_ATK, false, CELLS, NCHUNK, GW, INC, float, 1>);
-}
-
-// incremental: the in-place observation update (specialised board sizes only; others always write in full)
-template <typename F> static cudaError_t for_each_step_kernel(const td_handle *h, bool incremental, F f)
-{
-    switch (h->L) {
-    case 10:
-        return incremental ? for_each_kind<100, 32 / TD_GROUP_SMALL, TD_GROUP_SMALL, true>(f)
-                           : for_each_kind<100, 32 / TD_GROUP_SMALL, TD_GROUP_SMALL, false>(f);   // 32 live enemies
-    case 20: return incremental ? for_each_kind<400, 2, 32, true>(f) : for_each_kind<400, 2, 32, false>(f);
-    case 30: return incremental ? for_each_kind<900, 2, 32, true>(f) : for_each_kind<900, 2, 32, false>(f);
-    default: return for_each_kind<0, 2, 32, false>(f);
+    switch (kind) {
+    case TD_KIND_DEF:
+        if (scripted)
+            return multi ? td_step_kernel<TD_KIND_DEF, true, CELLS, NCHUNK, GW, INC, float, 1>
+                         : td_step_kernel<TD_KIND_DEF, false, CELLS, NCHUNK, GW, INC, float, 1>;
+        return multi ? td_step_kernel<TD_KIND_DEF, true, CELLS, NCHUNK, GW, INC> : td_step_kernel<TD_KIND_DEF, false, CELLS, NCHUNK, GW, INC>;
+    case TD_KIND_ATK:
+        return scripted ? td_step_kernel<TD_KIND_ATK, false, CELLS, NCHUNK, GW, INC, float, 1>
+                        : td_step_kernel<TD_KIND_ATK, false, CELLS, NCHUNK, GW, INC>;
+    default:
+        return multi ? td_step_kernel<TD_KIND_2P, true, CELLS, NCHUNK, GW, INC> : td_step_kernel<TD_KIND_2P, false, CELLS, NCHUNK, GW, INC>;
     }
 }
 
-// reduced-precision observation variants (td_step_io.obs_format): Discrete actions, full writes, boards 10 / 20 / 30
-template <int CELLS, int NCHUNK, class OT, typename F> static cudaError_t for_each_kind_fmt(F f)
+// reduced-precision observation kernels (td_step_io.obs_format): Discrete actions, full writes, opponent read at run time
+template <int CELLS, int NCHUNK, class OT> static StepKernel reduced_step_kernel(int kind)
 {
-    cudaError_t e;
-    if ((e = f(td_step_kernel<TD_KIND_DEF, false, CELLS, NCHUNK, 32, false, OT>)) != cudaSuccess) return e;
-    if ((e = f(td_step_kernel<TD_KIND_ATK, false, CELLS, NCHUNK, 32, false, OT>)) != cudaSuccess) return e;
-    return f(td_step_kernel<TD_KIND_2P, false, CELLS, NCHUNK, 32, false, OT>);
+    switch (kind) {
+    case TD_KIND_DEF: return td_step_kernel<TD_KIND_DEF, false, CELLS, NCHUNK, 32, false, OT>;
+    case TD_KIND_ATK: return td_step_kernel<TD_KIND_ATK, false, CELLS, NCHUNK, 32, false, OT>;
+    default: return td_step_kernel<TD_KIND_2P, false, CELLS, NCHUNK, 32, false, OT>;
+    }
 }
 
-template <class OT, typename F> static cudaError_t for_each_fmt_kernel(const td_handle *h, F f)
+// The step kernel for a board size L, an env kind, Discrete / multi-action, the in-place observation update, an
+// observation format (TD_OBS_F32 when no observation is written) and the opponent specialisation; NULL: none is
+// compiled.  10x10 boards hold at most 32 live enemies (one per lane), larger boards 64; other sizes take the
+// run-time-size kernels, which always write the observation in full.
+static StepKernel step_kernel(int L, int kind, bool multi, bool incremental, int obs_format, bool scripted)
 {
-    switch (h->L) {
-    case 10: return for_each_kind_fmt<100, 1, OT>(f);
-    case 20: return for_each_kind_fmt<400, 2, OT>(f);
-    case 30: return for_each_kind_fmt<900, 2, OT>(f);
-    default: return cudaErrorInvalidValue;
+    if (obs_format != TD_OBS_F32) {
+        if (multi) return nullptr;
+        const bool bf16 = obs_format == TD_OBS_BF16;
+        switch (L) {
+        case 10: return bf16 ? reduced_step_kernel<100, 1, __nv_bfloat16>(kind) : reduced_step_kernel<100, 1, uint8_t>(kind);
+        case 20: return bf16 ? reduced_step_kernel<400, 2, __nv_bfloat16>(kind) : reduced_step_kernel<400, 2, uint8_t>(kind);
+        case 30: return bf16 ? reduced_step_kernel<900, 2, __nv_bfloat16>(kind) : reduced_step_kernel<900, 2, uint8_t>(kind);
+        default: return nullptr;
+        }
+    }
+    switch (L) {
+    case 10:
+        return incremental ? f32_step_kernel<100, 32 / TD_GROUP_SMALL, TD_GROUP_SMALL, true>(kind, multi, scripted)
+                           : f32_step_kernel<100, 32 / TD_GROUP_SMALL, TD_GROUP_SMALL, false>(kind, multi, scripted);
+    case 20:
+        return incremental ? f32_step_kernel<400, 2, 32, true>(kind, multi, scripted) : f32_step_kernel<400, 2, 32, false>(kind, multi, scripted);
+    case 30:
+        return incremental ? f32_step_kernel<900, 2, 32, true>(kind, multi, scripted) : f32_step_kernel<900, 2, 32, false>(kind, multi, scripted);
+    default: return f32_step_kernel<0, 2, 32, false>(kind, multi, scripted);
+    }
+}
+
+// The observation writer (td_observe_kernel) for a board size and format; NULL: none is compiled (reduced precision:
+// boards 10 / 20 / 30 only).
+template <class OT> static const void *specialised_observe_kernel(int L)
+{
+    switch (L) {
+    case 10: return (const void *)td_observe_kernel<100, OT>;
+    case 20: return (const void *)td_observe_kernel<400, OT>;
+    case 30: return (const void *)td_observe_kernel<900, OT>;
+    default: return nullptr;
+    }
+}
+
+static const void *observe_kernel(int L, int obs_format)
+{
+    switch (obs_format) {
+    case TD_OBS_F32: {
+        const void *k = specialised_observe_kernel<float>(L);
+        return k ? k : (const void *)td_observe_kernel<0>;
+    }
+    case TD_OBS_BF16: return specialised_observe_kernel<__nv_bfloat16>(L);
+    case TD_OBS_U8: return specialised_observe_kernel<uint8_t>(L);
+    default: return nullptr;
     }
 }
 
@@ -372,8 +395,7 @@ extern "C" int td_create(const td_config *cfg, int env_kind, int map_size, int n
     td_handle *h = new (std::nothrow) td_handle();
     if (!h) return fail(nullptr, TD_E_ALLOC, "out of host memory");
     h->device = device; h->kind = env_kind; h->L = map_size; h->cells = map_size * map_size;
-    h->cells_pad = round16(h->cells); h->n_envs = n_envs;
-    h->n_maps = 0; h->map_stride = n_envs; h->difficulty = 1;
+    h->cells_pad = round16(h->cells); h->n_envs = n_envs; h->map_stride = n_envs;
     h->map_bytes = kMapHdrBytes + 2 * h->cells_pad;
     h->rng_cache_words = env_kind == TD_KIND_ATK ? kRngCacheAtk : kRngCacheDef;
     h->off_map6 = kOffRngCache + 4 * h->rng_cache_words;
@@ -390,37 +412,25 @@ extern "C" int td_create(const td_config *cfg, int env_kind, int map_size, int n
     if (env_kind != TD_KIND_DEF) scratch += TD_ROADS * TD_CLUSTER * 8;
     if (env_kind != TD_KIND_2P) scratch += kTwistStageBytes;
     h->smem_per_warp = h->record_bytes + scratch;
-    h->obs_synced = nullptr;
-    h->records = nullptr; h->maps = nullptr; h->mt = nullptr; h->stats = nullptr; h->stats_dev = nullptr;
-    h->opponent_seeded = false; h->steps = 0;
-    h->host_graph_clock = 0; h->host_stream = nullptr; h->host_chunks = 0; h->host_graph = 1;
-    h->step_smem_kb = 0; h->obs_smem_kb = 0; h->cfg_generation = 0; h->generic_kernels = false;
-    h->host_chain = false; h->host_first_chunk = -1; h->host_zero_copy = -1;
     td_config def;
     if (!cfg) { td_default_config(&def); cfg = &def; }
     int rc = validate_config(h, cfg);
     auto bail = [&](int code) { g_create_error = h->err; td_destroy(h); return code; };
     if (rc != TD_OK) return bail(rc);
     if ((e = cudaSetDevice(device)) != cudaSuccess) { h->err = cudaGetErrorString(e); return bail(TD_E_CUDA); }
-    size_t smem = smem_of(h);
-    const size_t step_smem = step_smem_bytes(h);
+    const size_t smem = smem_of(h), step_smem = step_smem_bytes(h);
     if (step_smem > 227 * 1024) { h->err = "map too large for shared memory"; return bail(TD_E_INVALID); }
-    if ((e = for_each_step_kernel(h, false, [&](auto kernel) { return allow_smem(kernel, step_smem); })) != cudaSuccess ||
-        (e = for_each_step_kernel(h, true, [&](auto kernel) { return allow_smem(kernel, step_smem); })) != cudaSuccess ||
-        ((h->L == 10 || h->L == 20 || h->L == 30) &&
-         ((e = for_each_fmt_kernel<__nv_bfloat16>(h, [&](auto kernel) { return allow_smem(kernel, step_smem); })) != cudaSuccess ||
-          (e = for_each_fmt_kernel<uint8_t>(h, [&](auto kernel) { return allow_smem(kernel, step_smem); })) != cudaSuccess ||
-          (e = allow_smem(td_observe_kernel<100, __nv_bfloat16>, smem)) != cudaSuccess ||
-          (e = allow_smem(td_observe_kernel<400, __nv_bfloat16>, smem)) != cudaSuccess ||
-          (e = allow_smem(td_observe_kernel<900, __nv_bfloat16>, smem)) != cudaSuccess ||
-          (e = allow_smem(td_observe_kernel<100, uint8_t>, smem)) != cudaSuccess ||
-          (e = allow_smem(td_observe_kernel<400, uint8_t>, smem)) != cudaSuccess ||
-          (e = allow_smem(td_observe_kernel<900, uint8_t>, smem)) != cudaSuccess)) ||
-        (e = allow_smem(td_reset_kernel, smem)) != cudaSuccess ||
-        (e = allow_smem(td_observe_kernel<0>, smem)) != cudaSuccess ||
-        (e = allow_smem(td_observe_kernel<100>, smem)) != cudaSuccess ||
-        (e = allow_smem(td_observe_kernel<400>, smem)) != cudaSuccess ||
-        (e = allow_smem(td_observe_kernel<900>, smem)) != cudaSuccess) {
+    // every kernel the handle can launch: the reset, and the observe and step kernels step_kernel / observe_kernel
+    // pick for its board size and env kind
+    auto allow = [&](auto kernel, size_t bytes) { if (kernel && e == cudaSuccess) e = allow_smem(kernel, bytes); };
+    allow(td_reset_kernel, smem);
+    for (int fmt : {TD_OBS_F32, TD_OBS_BF16, TD_OBS_U8}) {
+        allow(observe_kernel(h->L, fmt), smem);
+        for (bool multi : {false, true})
+            for (bool incremental : {false, true})
+                for (bool scripted : {false, true}) allow(step_kernel(h->L, env_kind, multi, incremental, fmt, scripted), step_smem);
+    }
+    if (e != cudaSuccess) {
         h->err = std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(e);
         return bail(TD_E_CUDA);
     }
@@ -650,6 +660,19 @@ extern "C" int td_get_opponent(td_handle *h, int first_env, int n, uint32_t *sta
     return TD_OK;
 }
 
+// A bf16 / u8 observation buffer: a known format, a board the reduced-precision kernels are compiled for, and an
+// address aligned for their stores.
+static int check_reduced_obs(td_handle *h, const char *who, int obs_format, const void *obs_dev)
+{
+    const std::string w(who);
+    if (obs_format != TD_OBS_BF16 && obs_format != TD_OBS_U8) return fail(h, TD_E_INVALID, w + ": unknown obs_format");
+    if (!(h->L == 10 || h->L == 20 || h->L == 30))
+        return fail(h, TD_E_INVALID, w + ": reduced-precision observations need a 10 / 20 / 30 board");
+    if (reinterpret_cast<uintptr_t>(obs_dev) & (obs_format == TD_OBS_BF16 ? 7 : 3))
+        return fail(h, TD_E_INVALID, w + ": obs_dev is not aligned for this obs_format");
+    return TD_OK;
+}
+
 static int check_io(td_handle *h, const td_step_io *io)
 {
     if (!io) return fail(h, TD_E_INVALID, "td_step: io is NULL");
@@ -662,11 +685,8 @@ static int check_io(td_handle *h, const td_step_io *io)
     if (io->opponent_dev && io->opponent_cluster_dev)
         return fail(h, TD_E_INVALID, "td_step: give opponent_dev or opponent_cluster_dev, not both");
     if (io->obs_format != TD_OBS_F32 && io->obs_dev) {
-        if (io->obs_format != TD_OBS_BF16 && io->obs_format != TD_OBS_U8) return fail(h, TD_E_INVALID, "td_step: unknown obs_format");
-        if (!(h->L == 10 || h->L == 20 || h->L == 30) || io->multi_action)
-            return fail(h, TD_E_INVALID, "td_step: reduced-precision observations need a 10 / 20 / 30 board and Discrete actions");
-        if (reinterpret_cast<uintptr_t>(io->obs_dev) & (io->obs_format == TD_OBS_BF16 ? 7 : 3))
-            return fail(h, TD_E_INVALID, "td_step: obs_dev is not aligned for this obs_format");
+        if (io->multi_action) return fail(h, TD_E_INVALID, "td_step: reduced-precision observations need Discrete actions");
+        return check_reduced_obs(h, "td_step", io->obs_format, io->obs_dev);
     }
     return TD_OK;
 }
@@ -700,20 +720,15 @@ static int launch_step(td_handle *h, const td_step_io *io, int begin, int count,
     const int wpc = step_warps_per_cta(h, incremental);
     const int per_cta = wpc * 32 / step_group_width(h);                  // game instances per CTA
     const int grid = (count + per_cta - 1) / per_cta, block = wpc * 32;
-    size_t smem = wpc == kWarpsPerCta ? step_smem_bytes(h) : (size_t)per_cta * h->smem_per_warp;
-    if (h->step_smem_kb > 0 && (size_t)h->step_smem_kb * 1024 > smem) {       // experiments (td_set_option)
-        smem = (size_t)h->step_smem_kb * 1024;
-        for_each_step_kernel(h, incremental, [&](auto kernel) { return allow_smem(kernel, smem); });
-    }
-    const bool reduced = io->obs_format != TD_OBS_F32 && io->obs_dev != nullptr;
-    const int want = reduced ? h->kind : step_variant(h, io);
-    int seen = 0;
-    auto launch = [&](auto kernel) {
-        if (seen++ != want) return cudaSuccess;
-        if (!t.graph) {
-            kernel<<<grid, block, smem, t.stream>>>(p);
-            return cudaGetLastError();
-        }
+    const size_t smem = wpc == kWarpsPerCta ? step_smem_bytes(h) : (size_t)per_cta * h->smem_per_warp;
+    const StepKernel kernel = step_kernel(h->L, h->kind, io->multi_action != 0, incremental,
+                                          io->obs_dev ? io->obs_format : TD_OBS_F32, scripted_lv1_on_device(h, io));
+    if (!kernel) return fail(h, TD_E_INVALID, "td_step: no step kernel is compiled for this configuration");
+    cudaError_t e;
+    if (!t.graph) {
+        kernel<<<grid, block, smem, t.stream>>>(p);
+        e = cudaGetLastError();
+    } else {
         void *args[] = {&p};
         cudaKernelNodeParams kp;
         memset(&kp, 0, sizeof(kp));
@@ -722,12 +737,9 @@ static int launch_step(td_handle *h, const td_step_io *io, int begin, int count,
         kp.blockDim = dim3(block);
         kp.sharedMemBytes = (unsigned)smem;
         kp.kernelParams = args;
-        return cudaGraphAddKernelNode(&t.node, t.graph, t.deps, t.n_deps, &kp);
-    };
-    cudaError_t le = !reduced ? for_each_step_kernel(h, incremental, launch)
-                     : io->obs_format == TD_OBS_BF16 ? for_each_fmt_kernel<__nv_bfloat16>(h, launch)
-                                                     : for_each_fmt_kernel<uint8_t>(h, launch);
-    if (le != cudaSuccess) return fail(h, TD_E_CUDA, std::string("td_step: ") + cudaGetErrorString(le));
+        e = cudaGraphAddKernelNode(&t.node, t.graph, t.deps, t.n_deps, &kp);
+    }
+    if (e != cudaSuccess) return fail(h, TD_E_CUDA, std::string("td_step: ") + cudaGetErrorString(e));
     return TD_OK;
 }
 
@@ -746,30 +758,33 @@ extern "C" int td_step(td_handle *h, const td_step_io *io, void *stream)
     return TD_OK;
 }
 
+// td_observe_kernel over the records [0, n) at records_dev (read only) into obs_dev, of a validated format
+static int launch_observe(td_handle *h, const char *who, const void *records_dev, int n, int obs_format, void *obs_dev,
+                          void *stream)
+{
+    StepParams p;
+    fill_params(h, p);
+    p.records = static_cast<uint8_t *>(const_cast<void *>(records_dev));
+    p.n_envs = n;
+    void *args[] = {&p, &obs_dev};
+    const cudaError_t e = cudaLaunchKernel(observe_kernel(h->L, obs_format), dim3((n + kWarpsPerCta - 1) / kWarpsPerCta),
+                                           dim3(kWarpsPerCta * 32), args, smem_of(h), (cudaStream_t)stream);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(h, TD_E_CUDA, std::string(who) + ": " + cudaGetErrorString(e));
+    }
+    return TD_OK;
+}
+
 extern "C" int td_observe(td_handle *h, float *obs_dev, void *stream)
 {
     if (!h) return TD_E_INVALID;
     if (!obs_dev) return fail(h, TD_E_INVALID, "td_observe: obs_dev is NULL");
     if (h->n_maps < 1) return fail(h, TD_E_STATE, "td_observe: upload maps and reset first");
     TD_CUDA(h, cudaSetDevice(h->device));
-    StepParams p;
-    fill_params(h, p);
-    const int grid = grid_of(h), block = kWarpsPerCta * 32;
-    size_t smem = smem_of(h);
-    if (h->obs_smem_kb > 0) {                                   // experiments (td_set_option)
-        smem = std::max(smem, (size_t)h->obs_smem_kb * 1024);
-        cudaFuncSetAttribute(td_observe_kernel<100>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    }
-    cudaStream_t s = (cudaStream_t)stream;
-    switch (h->L) {
-    case 10: td_observe_kernel<100><<<grid, block, smem, s>>>(p, obs_dev); break;
-    case 20: td_observe_kernel<400><<<grid, block, smem, s>>>(p, obs_dev); break;
-    case 30: td_observe_kernel<900><<<grid, block, smem, s>>>(p, obs_dev); break;
-    default: td_observe_kernel<0><<<grid, block, smem, s>>>(p, obs_dev); break;
-    }
+    const int rc = launch_observe(h, "td_observe", h->records, h->n_envs, TD_OBS_F32, obs_dev, stream);
     h->obs_synced = obs_dev;
-    TD_CUDA(h, cudaGetLastError());
-    return TD_OK;
+    return rc;
 }
 
 extern "C" int td_observe_as(td_handle *h, int obs_format, void *obs_dev, void *stream)
@@ -777,29 +792,11 @@ extern "C" int td_observe_as(td_handle *h, int obs_format, void *obs_dev, void *
     if (!h) return TD_E_INVALID;
     if (obs_format == TD_OBS_F32) return td_observe(h, static_cast<float *>(obs_dev), stream);
     if (!obs_dev) return fail(h, TD_E_INVALID, "td_observe_as: obs_dev is NULL");
-    if (obs_format != TD_OBS_BF16 && obs_format != TD_OBS_U8) return fail(h, TD_E_INVALID, "td_observe_as: unknown obs_format");
-    if (!(h->L == 10 || h->L == 20 || h->L == 30)) return fail(h, TD_E_INVALID, "td_observe_as: board sizes 10 / 20 / 30 only");
-    if (reinterpret_cast<uintptr_t>(obs_dev) & (obs_format == TD_OBS_BF16 ? 7 : 3)) return fail(h, TD_E_INVALID, "td_observe_as: obs_dev is not aligned");
+    const int rc = check_reduced_obs(h, "td_observe_as", obs_format, obs_dev);
+    if (rc != TD_OK) return rc;
     if (h->n_maps < 1) return fail(h, TD_E_STATE, "td_observe_as: upload maps and reset first");
     TD_CUDA(h, cudaSetDevice(h->device));
-    StepParams p;
-    fill_params(h, p);
-    const int grid = grid_of(h), block = kWarpsPerCta * 32;
-    const size_t smem = smem_of(h);
-    cudaStream_t s = (cudaStream_t)stream;
-    if (obs_format == TD_OBS_BF16) {
-        __nv_bfloat16 *o = static_cast<__nv_bfloat16 *>(obs_dev);
-        if (h->L == 10) td_observe_kernel<100, __nv_bfloat16><<<grid, block, smem, s>>>(p, o);
-        else if (h->L == 20) td_observe_kernel<400, __nv_bfloat16><<<grid, block, smem, s>>>(p, o);
-        else td_observe_kernel<900, __nv_bfloat16><<<grid, block, smem, s>>>(p, o);
-    } else {
-        uint8_t *o = static_cast<uint8_t *>(obs_dev);
-        if (h->L == 10) td_observe_kernel<100, uint8_t><<<grid, block, smem, s>>>(p, o);
-        else if (h->L == 20) td_observe_kernel<400, uint8_t><<<grid, block, smem, s>>>(p, o);
-        else td_observe_kernel<900, uint8_t><<<grid, block, smem, s>>>(p, o);
-    }
-    TD_CUDA(h, cudaGetLastError());
-    return TD_OK;
+    return launch_observe(h, "td_observe_as", h->records, h->n_envs, obs_format, obs_dev, stream);
 }
 
 // Compact snapshots (SURVEY 8(f) f4): the env records as they are, and observations rebuilt from them later.
@@ -818,22 +815,9 @@ extern "C" int td_observe_snapshot(td_handle *h, const void *records_dev, int n,
     if (!h) return TD_E_INVALID;
     if (!records_dev || !obs_dev || n < 1) return fail(h, TD_E_INVALID, "td_observe_snapshot: bad arguments");
     TD_CUDA(h, cudaSetDevice(h->device));
-    StepParams p;
-    fill_params(h, p);
-    p.records = static_cast<uint8_t *>(const_cast<void *>(records_dev));     // read-only in the observe kernel
-    p.n_envs = n;
-    const int grid = (n + kWarpsPerCta - 1) / kWarpsPerCta, block = kWarpsPerCta * 32;
-    const size_t smem = smem_of(h);
-    cudaStream_t s = (cudaStream_t)stream;
-    switch (h->L) {
-    case 10: td_observe_kernel<100><<<grid, block, smem, s>>>(p, obs_dev); break;
-    case 20: td_observe_kernel<400><<<grid, block, smem, s>>>(p, obs_dev); break;
-    case 30: td_observe_kernel<900><<<grid, block, smem, s>>>(p, obs_dev); break;
-    default: td_observe_kernel<0><<<grid, block, smem, s>>>(p, obs_dev); break;
-    }
+    const int rc = launch_observe(h, "td_observe_snapshot", records_dev, n, TD_OBS_F32, obs_dev, stream);
     if (obs_dev == h->obs_synced) h->obs_synced = nullptr;      // the buffer now shows the snapshot, not the live envs
-    TD_CUDA(h, cudaGetLastError());
-    return TD_OK;
+    return rc;
 }
 
 // One host-buffer step (td_step_host).  Inputs the step kernel can read from the caller's page-locked buffer
@@ -952,48 +936,59 @@ static std::vector<int> host_chunk_sizes(const td_handle *h, const HostPlan &pla
     return counts;
 }
 
-static int build_host_graph(td_handle *h, const td_step_io *io, const td_host_io *host, const HostPlan &plan, bool incremental,
-                            cudaGraphExec_t *exec_out)
+// The operations of one td_step_host call, chunk by chunk: input copies, the step kernel, output copies -- issued on
+// t.stream, or added to t.graph.  In the graph the output copies wait for their kernel; the kernels are chained
+// (each waits for its own input copies and the kernel before it), or -- plan.chain off -- independent branches that
+// start as soon as their own inputs are in, with the input copies of successive chunks following each other (chunk
+// order on the copy engine).
+static int issue_host_chunks(td_handle *h, const td_step_io *io, const td_host_io *host, const HostPlan &plan,
+                             bool incremental, LaunchTarget t)
 {
-    cudaGraph_t g = nullptr;
-    TD_CUDA(h, cudaGraphCreate(&g, 0));
-    auto bail = [&](int rc) { cudaGraphDestroy(g); return rc; };
-    std::vector<HostCopy> in, out;
+    auto copy = [&](const HostCopy &cp, cudaMemcpyKind dir, const cudaGraphNode_t *deps, size_t n_deps, cudaGraphNode_t *node) {
+        cudaError_t e = t.graph ? cudaGraphAddMemcpyNode1D(node, t.graph, deps, n_deps, cp.dst, cp.src, cp.bytes, dir)
+                                : cudaMemcpyAsync(cp.dst, cp.src, cp.bytes, dir, t.stream);
+        return e == cudaSuccess ? TD_OK : fail(h, TD_E_CUDA, std::string("td_step_host: copy: ") + cudaGetErrorString(e));
+    };
+    std::vector<HostCopy> &in = h->host_in, &out = h->host_out;
+    std::vector<cudaGraphNode_t> prev_copies, deps;
     cudaGraphNode_t prev_kernel = nullptr;
-    std::vector<cudaGraphNode_t> prev_copies;
-    int begin = 0;
+    int begin = 0, rc;
     for (int count : host_chunk_sizes(h, plan)) {
         host_chunk_copies(h, io, host, (size_t)begin, (size_t)count, in, out);
-        std::vector<cudaGraphNode_t> deps;
+        deps.clear();
         for (const HostCopy &cp : in) {
-            // input copies of successive chunks follow each other (chunk order on the copy engine); the kernels are
-            // chained too, or -- host_chain off -- independent branches that start as soon as their own inputs are in
-            cudaGraphNode_t n;
-            cudaError_t e = cudaGraphAddMemcpyNode1D(&n, g, plan.chain ? nullptr : prev_copies.data(), plan.chain ? 0 : prev_copies.size(),
-                                                     cp.dst, cp.src, cp.bytes, cudaMemcpyHostToDevice);
-            if (e != cudaSuccess) return bail(fail(h, TD_E_CUDA, std::string("td_step_host: memcpy node: ") + cudaGetErrorString(e)));
+            cudaGraphNode_t n = nullptr;
+            if ((rc = copy(cp, cudaMemcpyHostToDevice, plan.chain ? nullptr : prev_copies.data(), plan.chain ? 0 : prev_copies.size(), &n)) != TD_OK)
+                return rc;
             deps.push_back(n);
         }
         prev_copies = deps;
         if (prev_kernel && plan.chain) deps.push_back(prev_kernel);
-        LaunchTarget t;
-        t.graph = g;
         t.deps = deps.data();
         t.n_deps = deps.size();
-        int rc = launch_step(h, io, begin, count, t, incremental);
-        if (rc != TD_OK) return bail(rc);
+        if ((rc = launch_step(h, io, begin, count, t, incremental)) != TD_OK) return rc;
         for (const HostCopy &cp : out) {
-            cudaGraphNode_t n;
-            cudaError_t e = cudaGraphAddMemcpyNode1D(&n, g, &t.node, 1, cp.dst, cp.src, cp.bytes, cudaMemcpyDeviceToHost);
-            if (e != cudaSuccess) return bail(fail(h, TD_E_CUDA, std::string("td_step_host: memcpy node: ") + cudaGetErrorString(e)));
+            cudaGraphNode_t n = nullptr;
+            if ((rc = copy(cp, cudaMemcpyDeviceToHost, &t.node, 1, &n)) != TD_OK) return rc;
         }
         prev_kernel = t.node;
         begin += count;
     }
-    cudaError_t e = cudaGraphInstantiate(exec_out, g, 0);
-    cudaGraphDestroy(g);
-    if (e != cudaSuccess) return fail(h, TD_E_CUDA, std::string("td_step_host: cudaGraphInstantiate: ") + cudaGetErrorString(e));
     return TD_OK;
+}
+
+static int build_host_graph(td_handle *h, const td_step_io *io, const td_host_io *host, const HostPlan &plan, bool incremental,
+                            cudaGraphExec_t *exec_out)
+{
+    LaunchTarget t;
+    TD_CUDA(h, cudaGraphCreate(&t.graph, 0));
+    int rc = issue_host_chunks(h, io, host, plan, incremental, t);
+    if (rc == TD_OK) {
+        const cudaError_t e = cudaGraphInstantiate(exec_out, t.graph, 0);
+        if (e != cudaSuccess) rc = fail(h, TD_E_CUDA, std::string("td_step_host: cudaGraphInstantiate: ") + cudaGetErrorString(e));
+    }
+    cudaGraphDestroy(t.graph);
+    return rc;
 }
 
 extern "C" int td_step_host(td_handle *h, const td_step_io *io, const td_host_io *host, void *stream)
@@ -1105,19 +1100,11 @@ extern "C" int td_step_host(td_handle *h, const td_step_io *io, const td_host_io
         hit->used = ++h->host_graph_clock;
         TD_CUDA(h, cudaGraphLaunch(hit->exec, s));
     } else {
-        // plain stream launches, chunk by chunk (pageable host memory or TD_OPT_HOST_GRAPH = 0)
-        std::vector<HostCopy> &in = h->host_in, &out = h->host_out;
-        int begin = 0;
-        for (int count : host_chunk_sizes(h, host_plan(h, io, host, false))) {
-            host_chunk_copies(h, io, host, (size_t)begin, (size_t)count, in, out);
-            for (const HostCopy &cp : in) TD_CUDA(h, cudaMemcpyAsync(cp.dst, cp.src, cp.bytes, cudaMemcpyHostToDevice, s));
-            LaunchTarget t;
-            t.stream = s;
-            rc = launch_step(h, io, begin, count, t, incremental);
-            if (rc != TD_OK) return rc;
-            for (const HostCopy &cp : out) TD_CUDA(h, cudaMemcpyAsync(cp.dst, cp.src, cp.bytes, cudaMemcpyDeviceToHost, s));
-            begin += count;
-        }
+        // plain stream launches (pageable host memory or TD_OPT_HOST_GRAPH = 0)
+        LaunchTarget t;
+        t.stream = s;
+        rc = issue_host_chunks(h, io, host, host_plan(h, io, host, false), incremental, t);
+        if (rc != TD_OK) return rc;
     }
     h->obs_synced = io->obs_format == TD_OBS_F32 ? io->obs_dev : nullptr;
     h->steps += h->n_envs;
@@ -1141,14 +1128,6 @@ extern "C" int td_set_option(td_handle *h, int option, int value)
         h->host_chunks = value;
         return TD_OK;
     case TD_OPT_HOST_GRAPH: h->host_graph = value != 0; return TD_OK;
-    case TD_OPT_STEP_SMEM_KB:
-        if (value < 0 || value > 227) return fail(h, TD_E_INVALID, "td_set_option: shared memory out of range");
-        h->step_smem_kb = value;
-        return TD_OK;
-    case TD_OPT_OBS_SMEM_KB:
-        if (value < 0 || value > 227) return fail(h, TD_E_INVALID, "td_set_option: shared memory out of range");
-        h->obs_smem_kb = value;
-        return TD_OK;
     case TD_OPT_HOST_CHAIN:
         h->host_chain = value != 0;
         h->cfg_generation += 1;      // cached host-step graphs were built with the other shape

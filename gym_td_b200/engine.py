@@ -18,7 +18,7 @@ CAP_TOWERS, CAP_ENEMIES = 32, 64
 KIND_DEF, KIND_ATK, KIND_2P = 0, 1, 2
 KINDS = {"def": KIND_DEF, "atk": KIND_ATK, "2p": KIND_2P}
 OBS_FORMATS = {"f32": 0, "bf16": 1, "u8": 2}
-OPTIONS = {"host_chunks": 1, "host_graph": 2, "step_smem_kb": 3, "obs_smem_kb": 4, "generic_kernels": 5, "host_chain": 6, "host_first_chunk": 7, "host_zero_copy": 8}
+OPTIONS = {"host_chunks": 1, "host_graph": 2, "generic_kernels": 5, "host_chain": 6, "host_first_chunk": 7, "host_zero_copy": 8}
 
 _TABLES_F64 = ["enemy_LP", "enemy_speed", "enemy_defense", "enemy_cost", "tower_attack", "tower_cost",
                "tower_attack_interval"]
@@ -304,7 +304,7 @@ class Engine(object):
         self._check(self._lib.td_set_map_stride(self._h, int(stride)))
 
     def set_option(self, option, value):
-        """Tuning knobs of the handle (TD_OPT_* of td_b200.h): "host_chunks", "host_graph", "step_smem_kb", "obs_smem_kb", "generic_kernels"."""
+        """Tuning knobs of the handle (TD_OPT_* of td_b200.h): "host_chunks", "host_graph", "generic_kernels", "host_chain", "host_first_chunk", "host_zero_copy"."""
         self._check(self._lib.td_set_option(self._h, OPTIONS[option] if isinstance(option, str) else int(option), int(value)))
 
     def set_difficulty(self, difficulty):

@@ -323,8 +323,7 @@ int td_step_host(td_handle *h, const td_step_io *io, const td_host_io *host, voi
 /* tuning knobs of a handle (no environment variables are read anywhere in the library) */
 enum { TD_OPT_HOST_CHUNKS = 1,   /* td_step_host: chunks the batch is cut into; 0 = automatic (4 from 8,192 envs on) */
        TD_OPT_HOST_GRAPH = 2,    /* td_step_host: 1 = graph launch (default), 0 = plain stream launches */
-       TD_OPT_STEP_SMEM_KB = 3,  /* experiments: minimum dynamic shared memory of a step CTA (lowers residency) */
-       TD_OPT_OBS_SMEM_KB = 4,   /* experiments: the same for td_observe */
+       /* 3 and 4 are retired (former shared-memory experiments) and rejected; do not reuse them */
        TD_OPT_GENERIC_KERNELS = 5, /* 1 = never pick the step kernels specialised on the default scripted opponent
                                     (level 1 on the device generator); results are identical, for A/B runs and tests */
        TD_OPT_HOST_CHAIN = 6,    /* td_step_host graph with > 1 chunk: 0 = independent branches, each starts when its own
