@@ -32,7 +32,7 @@ def up_to_date():
 def build(force=False, verbose=False):
     if not force and up_to_date():
         return OUT
-    extra = os.environ.get("TD_NVCC_EXTRA", "").split()      # experiments, e.g. -DTD_MIN_BLOCKS=6
+    extra = os.environ.get("TD_NVCC_EXTRA", "").split()      # extra nvcc flags, e.g. -DTD_DEBUG_BOUNDS
     out = os.environ.get("TD_BUILD_OUT", OUT)                # experiments: a variant library next to the default
     cmd = [nvcc_path()] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-o", out] + \
           [os.path.join(CSRC, s) for s in SOURCES]

@@ -1,5 +1,5 @@
 // td_common.cuh -- shared definitions of the step kernels: record layout, derived config, kernel parameters, the
-// per-warp context over its shared-memory slice, group primitives, and the env record load / store / reset.
+// per-warp context over its shared-memory slice, and the env record load / store / reset.
 // Part of the kernel set described in td_kernels.cuh.
 #pragma once
 #include "../../include/td_b200.h"
@@ -7,32 +7,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-// Observation store flavour (experiments): 0 = st.global.cs (streaming), 1 = plain st.global, 2 = st.global.wt
-#ifndef TD_STORE_MODE
-#define TD_STORE_MODE 1
-#endif
-#if TD_STORE_MODE == 0
-#define TD_ST(p, v) __stcs((p), (v))
-#elif TD_STORE_MODE == 1
-#define TD_ST(p, v) (*(p) = (v))
-#elif TD_STORE_MODE == 2
-#define TD_ST(p, v) __stwt((p), (v))
-#else
-// L2 evict_first policy on the observation stream: the env records keep their place in L2 (tools/storebench_l2.cu)
-__device__ __forceinline__ void td_st_first(float4 *a, float4 v)
-{
-    unsigned long long pol;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-    asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1,%2,%3,%4}, %5;" ::"l"(a), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w), "l"(pol) : "memory");
-}
-__device__ __forceinline__ void td_st_first(float *a, float v)
-{
-    unsigned long long pol;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-    asm volatile("st.global.L2::cache_hint.f32 [%0], %1, %2;" ::"l"(a), "f"(v), "l"(pol) : "memory");
-}
-#define TD_ST(p, v) td_st_first((p), (v))
-#endif
 // Debug build (-DTD_DEBUG_BOUNDS): index invariants are checked on the device and a violation sets the sticky
 // flag bit 2 of the env, which TDVecEnv.stats() / the parity tests surface.  (compute-sanitizer is closed on
 // the B200 pool, so this is the memory-safety net next to the bit-exact parity runs.)
@@ -41,21 +15,16 @@ __device__ __forceinline__ void td_st_first(float *a, float v)
 #else
 #define TD_CHECK(w, cond) do { } while (0)
 #endif
-#ifndef TD_WARPS_PER_CTA
-#define TD_WARPS_PER_CTA 4
-#endif
-// Leading bytes of every env record that are loaded with an L2 evict_last policy (0 = none; >= 4096 = the whole
-// speculative load).  See DESIGN.md 7.2(c).
-#ifndef TD_L2_KEEP_BYTES
-#define TD_L2_KEEP_BYTES 0
-#endif
 
 
 namespace td {
 
 
-constexpr int kWarpsPerCta = TD_WARPS_PER_CTA;
+// One warp advances one env: every lane loop of the kernels strides by kLanes, and the warp intrinsics run on kFull.
+constexpr int kLanes = 32;
 constexpr unsigned kFull = 0xffffffffu;
+// Warps per CTA of the full-write step, reset and observe kernels (td_engine.cu: step_warps_per_cta).
+constexpr int kWarpsPerCta = 4;
 // Env record in HBM (mirrored byte for byte in the warp's shared-memory slice):
 //   [ td_env_header 64 | opponent word cache 64 | map6 cells_pad | static map (MapHdr 16, cells, dist) |
 //     towers 32 x 16 | enemies 64 x 24 ]
@@ -75,14 +44,12 @@ constexpr int kTwistStageBytes = kMtWords * 4;   // staging area of the generato
 // defender env, 11-13 in the attacker env whose scripted defender keeps building; live enemies p99 = 6): 12 towers
 // and 8 enemies cover almost every env and read 256 B less per env-step than 16 / 16 (def-small 0.2156 -> 0.2132 ms,
 // atk-small 0.2435 -> 0.2397 ms; 8 / 8 is best for def-small alone, 0.2126 ms, and neutral for atk-small).
-#ifndef TD_SPEC_TOWERS
-#define TD_SPEC_TOWERS 12
-#endif
-#ifndef TD_SPEC_ENEMIES
-#define TD_SPEC_ENEMIES 8
-#endif
-constexpr int kSpecTowers = TD_SPEC_TOWERS;     // speculatively staged list prefixes
-constexpr int kSpecEnemies = TD_SPEC_ENEMIES;
+constexpr int kSpecTowers = 12;
+constexpr int kSpecEnemies = 8;
+
+// Live enemies a step kernel holds on a board of side L: one per lane on 10x10 boards (one register chunk in
+// board_step), TD_CAP_ENEMIES (two chunks) on every other board.  td_set_state refuses records above it.
+__host__ __device__ constexpr int step_enemy_cap(int L) { return L == 10 ? kLanes : TD_CAP_ENEMIES; }
 
 // Derived constant tables (uploaded by td_set_config).
 struct DevConfig {
@@ -139,21 +106,16 @@ struct StepParams {
 
 // CELLS > 0: board size known at compile time -> every pointer into the slice is base + constant.
 // CELLS == 0: layout read from the kernel parameters (constant bank).
-// GW = lanes per game instance: 32 (one warp per env) or 16 (two envs per warp: the uniform bookkeeping
-// of both is issued once, and twice as many envs are in flight per SM at the same warp count).
-template <int CELLS, int GW, int RC = 0>
+template <int CELLS, int RC = 0>
 struct Ctx {
     static constexpr int kCells = CELLS;
-    static constexpr int G = GW;
     static constexpr int kRngWords = RC;
-    unsigned gmask;            // the warp lanes of this env's group
-    int gbase;                 // first warp lane of the group
     static constexpr int kL = CELLS == 100 ? 10 : CELLS == 400 ? 20 : CELLS == 900 ? 30 : 0;
     static constexpr int kPad = (CELLS + 15) & ~15;
     uint8_t *slice;            // the warp's shared-memory slice: [record | scratch]
     const StepParams *pp;
-    int lane, ecap;            // lane = index inside the group
-    // uniform copies of hot header fields (identical in all lanes of the group)
+    int lane, ecap;
+    // uniform copies of hot header fields (identical in all lanes of the warp)
     double cost_def, cost_atk;
     int nt, ne, base_LP, steps, def_cd, atk_cd, fail, flags;
     // opponent generator cursor
@@ -200,71 +162,39 @@ struct Ctx {
     }
 };
 
-// group-level primitives: ballots are returned relative to the group (bit 0 = group lane 0)
-template <class W> __device__ __forceinline__ unsigned gballot(const W &w, bool pred)
-{
-    const unsigned b = __ballot_sync(w.gmask, pred);
-    if (W::G == 32) return b;
-    return (b >> w.gbase) & 0xffffu;
-}
-template <class W, class T> __device__ __forceinline__ T gshfl(const W &w, T v, int src)
-{
-    return __shfl_sync(w.gmask, v, src, W::G);
-}
-template <class W> __device__ __forceinline__ bool gall(const W &w, bool pred) { return __all_sync(w.gmask, pred); }
-template <class W> __device__ __forceinline__ bool gany(const W &w, bool pred) { return __any_sync(w.gmask, pred); }
-template <class W> __device__ __forceinline__ void gsync(const W &w) { __syncwarp(w.gmask); }
-
 // n16 <= MAXN int4 with a compile-time bound: one predicated load/store pair per pass instead of a loop.
-template <int MAXN, int G>
+template <int MAXN>
 __device__ __forceinline__ void copy16_upto(void *dst, const void *src, int n16, int lane)
 {
     int4 *d = reinterpret_cast<int4 *>(dst);
     const int4 *s = reinterpret_cast<const int4 *>(src);
 #pragma unroll
-    for (int k = 0; k < (MAXN + G - 1) / G; ++k) {
-        const int q = lane + G * k;
+    for (int k = 0; k < (MAXN + kLanes - 1) / kLanes; ++k) {
+        const int q = lane + kLanes * k;
         if (q < n16) d[q] = s[q];
     }
 }
 
-__device__ __forceinline__ void warp_copy16(void *dst, const void *src, int n16, int lane, int stride)
+__device__ __forceinline__ void warp_copy16(void *dst, const void *src, int n16, int lane)
 {
     int4 *d = reinterpret_cast<int4 *>(dst);
     const int4 *s = reinterpret_cast<const int4 *>(src);
-    for (int q = lane; q < n16; q += stride) d[q] = s[q];
+    for (int q = lane; q < n16; q += kLanes) d[q] = s[q];
 }
 
 // global -> shared, 16 bytes per lane per instruction, asynchronous (LDGSTS): every segment of a stage
 // is in flight at once and no register is held while the data travels.
-// The same with an L2 evict_last policy on units [0, keep16): those lines keep their place in L2 under the observation
-// write stream (tools/storebench_l2.cu: lines brought in evict_last stay resident, later plain hits keep them).
-__device__ __forceinline__ void async_copy16_keep(void *smem_dst, const void *gmem_src, int n16, int keep16, int lane, int stride)
+__device__ __forceinline__ void async_copy16(void *smem_dst, const void *gmem_src, int n16, int lane)
 {
     const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
     const char *s = reinterpret_cast<const char *>(gmem_src);
-    unsigned long long pol;
-    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-    for (int q = lane; q < n16; q += stride) {
-        if (q < keep16)
-            asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0], [%1], 16, %2;" ::"r"(d + 16u * q), "l"(s + 16 * q), "l"(pol) : "memory");
-        else
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d + 16u * q), "l"(s + 16 * q) : "memory");
-    }
-}
-
-__device__ __forceinline__ void async_copy16(void *smem_dst, const void *gmem_src, int n16, int lane, int stride)
-{
-    const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
-    const char *s = reinterpret_cast<const char *>(gmem_src);
-    for (int q = lane; q < n16; q += stride)
+    for (int q = lane; q < n16; q += kLanes)
         asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d + 16u * q), "l"(s + 16 * q) : "memory");
 }
-template <class W>
-__device__ __forceinline__ void async_wait_all(const W &w)
+__device__ __forceinline__ void async_wait_all()
 {
     asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
-    gsync(w);
+    __syncwarp();
 }
 
 template <class W>
@@ -272,10 +202,7 @@ __device__ __forceinline__ void ctx_bind(W &w, uint8_t *slice, const StepParams 
 {
     w.slice = slice;
     w.pp = &p;
-    const int wl = threadIdx.x & 31;
-    w.lane = wl & (W::G - 1);
-    w.gbase = wl - w.lane;
-    w.gmask = W::G == 32 ? kFull : (0xffffu << w.gbase);
+    w.lane = threadIdx.x & 31;
     w.ecap = TD_CAP_ENEMIES;
     w.mt = nullptr;
     w.mt_pos = 0;
@@ -288,7 +215,7 @@ __device__ __forceinline__ void ctx_bind(W &w, uint8_t *slice, const StepParams 
 template <class W>
 __device__ __forceinline__ void load_static_map(W &w, const StepParams &p, int map_id)
 {
-    async_copy16(w.mh(), p.maps + (size_t)map_id * w.map_bytes(), w.map_bytes() >> 4, w.lane, W::G);
+    async_copy16(w.mh(), p.maps + (size_t)map_id * w.map_bytes(), w.map_bytes() >> 4, w.lane);
     w.static_dirty = true;
 }
 
@@ -336,16 +263,8 @@ __device__ __forceinline__ void push_header(W &w)
 template <class W>
 __device__ __forceinline__ void issue_env_load(W &w, const uint8_t *rec)
 {
-#if TD_L2_KEEP_BYTES > 0
-    async_copy16_keep(w.slice, rec, (w.off_towers() + kSpecTowers * kTowerBytes) >> 4, TD_L2_KEEP_BYTES >> 4, w.lane, W::G);
-#else
-    async_copy16(w.slice, rec, (w.off_towers() + kSpecTowers * kTowerBytes) >> 4, w.lane, W::G);
-#endif
-#if TD_L2_KEEP_BYTES >= 4096
-    async_copy16_keep(w.en(), rec + w.off_enemies(), (kSpecEnemies * kEnemyBytes) >> 4, 4096, w.lane, W::G);
-#else
-    async_copy16(w.en(), rec + w.off_enemies(), (kSpecEnemies * kEnemyBytes) >> 4, w.lane, W::G);
-#endif
+    async_copy16(w.slice, rec, (w.off_towers() + kSpecTowers * kTowerBytes) >> 4, w.lane);
+    async_copy16(w.en(), rec + w.off_enemies(), (kSpecEnemies * kEnemyBytes) >> 4, w.lane);
     asm volatile("cp.async.commit_group;" ::: "memory");
 }
 
@@ -357,11 +276,11 @@ __device__ __forceinline__ void finish_env_load(W &w, const StepParams &p, const
     w.mt = mt_base;
     if (__builtin_expect(w.nt > kSpecTowers || w.ne > kSpecEnemies, 0)) {
         if (w.nt > kSpecTowers)
-            async_copy16(w.tw() + kSpecTowers, rec + w.off_towers() + kSpecTowers * kTowerBytes, w.nt - kSpecTowers, w.lane, W::G);
+            async_copy16(w.tw() + kSpecTowers, rec + w.off_towers() + kSpecTowers * kTowerBytes, w.nt - kSpecTowers, w.lane);
         if (w.ne > kSpecEnemies)
             async_copy16(w.en() + kSpecEnemies, rec + w.off_enemies() + kSpecEnemies * kEnemyBytes,
-                         ((w.ne - kSpecEnemies) * 3 + 1) >> 1, w.lane, W::G);
-        async_wait_all(w);
+                         ((w.ne - kSpecEnemies) * 3 + 1) >> 1, w.lane);
+        async_wait_all();
     }
 }
 
@@ -369,7 +288,7 @@ template <class W>
 __device__ __forceinline__ void load_env(W &w, const StepParams &p, const uint8_t *rec, uint32_t *mt_base = nullptr)
 {
     issue_env_load(w, rec);
-    async_wait_all(w);
+    async_wait_all();
     finish_env_load(w, p, rec, mt_base);
 }
 
@@ -377,53 +296,35 @@ __device__ __forceinline__ void load_env(W &w, const StepParams &p, const uint8_
 // UNROLLED: predicated single-pass copies instead of loops -- 45 fewer instructions per env-step.  Measured on
 // B200: attacker env 0.291 -> 0.273 ms, in-place observation update (def-small) 0.191 -> 0.167 ms, but the
 // full-write defender step 0.2175 -> 0.2220 ms (same box, twice), so the caller chooses per kernel variant.
-// List write-back granularity (experiment): 1 = whole 32-byte sectors (the dead slot behind an odd list end goes back
-// as zeros), so that no partial-sector write reaches the ECC-protected HBM as a read-modify-write.  Measured on
-// B200: no difference (def-small 0.2160 vs 0.2158 ms, atk-small 0.2365 vs 0.2379) -- L2 merges them; off.
-#ifndef TD_WB_SECTORS
-#define TD_WB_SECTORS 0
-#endif
-#if TD_WB_SECTORS
-#define TD_WB_ROUND(n16) (((n16) + 1) & ~1)
-#else
-#define TD_WB_ROUND(n16) (n16)
-#endif
 template <bool UNROLLED = false, class W>
 __device__ __forceinline__ void store_env(W &w, const StepParams &p, uint8_t *rec, bool map6_dirty, bool push = true)
 {
     if (push) push_header(w);
-#if TD_WB_SECTORS
-    if (w.lane == 0) {          // the dead slot that rides along in the last sector goes back as zeros (deterministic)
-        const int e16 = (w.ne * 3 + 1) >> 1;
-        if (w.nt & 1) reinterpret_cast<int4 *>(w.tw())[w.nt] = make_int4(0, 0, 0, 0);
-        if (e16 & 1) reinterpret_cast<int4 *>(w.en())[e16] = make_int4(0, 0, 0, 0);
-    }
-#endif
-    gsync(w);
+    __syncwarp();
     const int head = w.static_dirty ? w.off_towers() : (map6_dirty ? w.off_static() : w.hdr_bytes());
     // the word cache block [kOffRngCache, hdr_bytes) goes back only when it was refilled
     const int skip_lo = w.cache_dirty ? 0 : (kOffRngCache >> 4), skip_hi = w.cache_dirty ? 0 : (w.hdr_bytes() >> 4);
     if (!UNROLLED) {
-        for (int q = w.lane; q < (head >> 4); q += W::G)
+        for (int q = w.lane; q < (head >> 4); q += kLanes)
             if (q < skip_lo || q >= skip_hi) reinterpret_cast<int4 *>(rec)[q] = reinterpret_cast<const int4 *>(w.slice)[q];
-        warp_copy16(rec + w.off_towers(), w.tw(), TD_WB_ROUND(w.nt), w.lane, W::G);
-        warp_copy16(rec + w.off_enemies(), w.en(), TD_WB_ROUND((w.ne * 3 + 1) >> 1), w.lane, W::G);
+        warp_copy16(rec + w.off_towers(), w.tw(), w.nt, w.lane);
+        warp_copy16(rec + w.off_enemies(), w.en(), (w.ne * 3 + 1) >> 1, w.lane);
         return;
     }
     if (W::kCells > 0 && W::kRngWords > 0) {
         constexpr int kHeadMax = (kOffRngCache + 4 * W::kRngWords + 3 * W::kPad + kMapHdrBytes) / 16;   // = off_towers / 16
 #pragma unroll
-        for (int k = 0; k < (kHeadMax + W::G - 1) / W::G; ++k) {
-            const int q = w.lane + W::G * k;
+        for (int k = 0; k < (kHeadMax + kLanes - 1) / kLanes; ++k) {
+            const int q = w.lane + kLanes * k;
             if (q < (head >> 4) && (q < skip_lo || q >= skip_hi))
                 reinterpret_cast<int4 *>(rec)[q] = reinterpret_cast<const int4 *>(w.slice)[q];
         }
     } else {
-        for (int q = w.lane; q < (head >> 4); q += W::G)
+        for (int q = w.lane; q < (head >> 4); q += kLanes)
             if (q < skip_lo || q >= skip_hi) reinterpret_cast<int4 *>(rec)[q] = reinterpret_cast<const int4 *>(w.slice)[q];
     }
-    copy16_upto<TD_CAP_TOWERS, W::G>(rec + w.off_towers(), w.tw(), TD_WB_ROUND(w.nt), w.lane);
-    copy16_upto<(TD_CAP_ENEMIES * 3 + 1) / 2, W::G>(rec + w.off_enemies(), w.en(), TD_WB_ROUND((w.ne * 3 + 1) >> 1), w.lane);
+    copy16_upto<TD_CAP_TOWERS>(rec + w.off_towers(), w.tw(), w.nt, w.lane);
+    copy16_upto<(TD_CAP_ENEMIES * 3 + 1) / 2>(rec + w.off_enemies(), w.en(), (w.ne * 3 + 1) >> 1, w.lane);
 }
 
 // TDGymBasic.reset (:37-55) + TDBoard.__init__ (:63-79): fresh episode on map `map_id`.
@@ -432,11 +333,11 @@ __device__ __forceinline__ void reset_env(W &w, const StepParams &p, int map_id,
 {
     const DevConfig &cc = w.pp->cfg;
     if (reload_map) {
-        gsync(w);
+        __syncwarp();
         load_static_map(w, p, map_id);
-        async_wait_all(w);
+        async_wait_all();
     }
-    for (int q = w.lane; q < (w.cells_pad() >> 2); q += W::G) {
+    for (int q = w.lane; q < (w.cells_pad() >> 2); q += kLanes) {
         uint32_t c4 = reinterpret_cast<const uint32_t *>(w.cells())[q];
         reinterpret_cast<uint32_t *>(w.map6())[q] = c4 & 0x01010101u;           // map[6] = 1 on road cells
     }
@@ -457,7 +358,7 @@ __device__ __forceinline__ void reset_env(W &w, const StepParams &p, int map_id,
         w.hdr()->ep_kills_hi = 0;
         w.hdr()->ep_leaks_hi = 0;
     }
-    gsync(w);
+    __syncwarp();
 }
 
 } // namespace td

@@ -251,14 +251,6 @@ static void fill_params(const td_handle *h, StepParams &p)
 static int grid_of(const td_handle *h) { return (h->n_envs + kWarpsPerCta - 1) / kWarpsPerCta; }
 static size_t smem_of(const td_handle *h) { return (size_t)kWarpsPerCta * h->smem_per_warp; }
 
-#ifndef TD_GROUP_SMALL
-#define TD_GROUP_SMALL 32     // lanes per game instance on 10x10 boards.  16 (two instances per warp) is
-                              // correct and makes the rules 10 % faster, but the full step 6 % slower on B200:
-                              // twice as many open observation streams per SM lower the store efficiency.
-#endif
-
-static int step_group_width(const td_handle *h) { return h->L == 10 ? TD_GROUP_SMALL : 32; }
-
 // Dynamic shared memory of one step CTA.  Boards whose observation is >= 128 KB ask for at least 75 KB so that
 // three CTAs (12 warps = 12 open observation streams) share an SM instead of six: HBM write efficiency falls
 // with the number of long streams written side by side (tools/storebench_sized.cu, test F: 162 KB regions at
@@ -267,9 +259,7 @@ static bool large_observation(const td_handle *h) { return (size_t)TD_NCHANNELS 
 
 static size_t step_smem_bytes(const td_handle *h)
 {
-    size_t bytes = (size_t)(kWarpsPerCta * 32 / step_group_width(h)) * h->smem_per_warp;
-    if (large_observation(h)) bytes = std::max(bytes, (size_t)75 * 1024);
-    return bytes;
+    return large_observation(h) ? std::max(smem_of(h), (size_t)75 * 1024) : smem_of(h);
 }
 
 // Warps per step CTA.  The full-write kernels are insensitive to it (1 / 2 / 4 warps: def-small 0.2131 / 0.2129 /
@@ -278,7 +268,7 @@ static size_t step_smem_bytes(const td_handle *h)
 static int step_warps_per_cta(const td_handle *h, bool incremental)
 {
     // (10x10 boards only: at 20x20 it changes nothing, 0.1921 vs 0.1916 ms)
-    return incremental && h->L == 10 && step_group_width(h) == 32 ? 1 : kWarpsPerCta;
+    return incremental && h->L == 10 ? 1 : kWarpsPerCta;
 }
 
 // The scripted opponent of level 1 draws from the device generator and no host-resolved opponent input is set:
@@ -294,57 +284,55 @@ using StepKernel = void (*)(StepParams);
 
 // float32 observation kernels of one board specialisation.  `scripted`: the default scripted opponent (level 1 on
 // the device generator) known at compile time, for the defender and the attacker env.
-template <int CELLS, int NCHUNK, int GW, bool INC> static StepKernel f32_step_kernel(int kind, bool multi, bool scripted)
+template <int CELLS, bool INC> static StepKernel f32_step_kernel(int kind, bool multi, bool scripted)
 {
     switch (kind) {
     case TD_KIND_DEF:
         if (scripted)
-            return multi ? td_step_kernel<TD_KIND_DEF, true, CELLS, NCHUNK, GW, INC, float, 1>
-                         : td_step_kernel<TD_KIND_DEF, false, CELLS, NCHUNK, GW, INC, float, 1>;
-        return multi ? td_step_kernel<TD_KIND_DEF, true, CELLS, NCHUNK, GW, INC> : td_step_kernel<TD_KIND_DEF, false, CELLS, NCHUNK, GW, INC>;
+            return multi ? td_step_kernel<TD_KIND_DEF, true, CELLS, INC, float, 1>
+                         : td_step_kernel<TD_KIND_DEF, false, CELLS, INC, float, 1>;
+        return multi ? td_step_kernel<TD_KIND_DEF, true, CELLS, INC> : td_step_kernel<TD_KIND_DEF, false, CELLS, INC>;
     case TD_KIND_ATK:
-        return scripted ? td_step_kernel<TD_KIND_ATK, false, CELLS, NCHUNK, GW, INC, float, 1>
-                        : td_step_kernel<TD_KIND_ATK, false, CELLS, NCHUNK, GW, INC>;
+        return scripted ? td_step_kernel<TD_KIND_ATK, false, CELLS, INC, float, 1>
+                        : td_step_kernel<TD_KIND_ATK, false, CELLS, INC>;
     default:
-        return multi ? td_step_kernel<TD_KIND_2P, true, CELLS, NCHUNK, GW, INC> : td_step_kernel<TD_KIND_2P, false, CELLS, NCHUNK, GW, INC>;
+        return multi ? td_step_kernel<TD_KIND_2P, true, CELLS, INC> : td_step_kernel<TD_KIND_2P, false, CELLS, INC>;
     }
 }
 
 // reduced-precision observation kernels (td_step_io.obs_format): Discrete actions, full writes, opponent read at run time
-template <int CELLS, int NCHUNK, class OT> static StepKernel reduced_step_kernel(int kind)
+template <int CELLS, class OT> static StepKernel reduced_step_kernel(int kind)
 {
     switch (kind) {
-    case TD_KIND_DEF: return td_step_kernel<TD_KIND_DEF, false, CELLS, NCHUNK, 32, false, OT>;
-    case TD_KIND_ATK: return td_step_kernel<TD_KIND_ATK, false, CELLS, NCHUNK, 32, false, OT>;
-    default: return td_step_kernel<TD_KIND_2P, false, CELLS, NCHUNK, 32, false, OT>;
+    case TD_KIND_DEF: return td_step_kernel<TD_KIND_DEF, false, CELLS, false, OT>;
+    case TD_KIND_ATK: return td_step_kernel<TD_KIND_ATK, false, CELLS, false, OT>;
+    default: return td_step_kernel<TD_KIND_2P, false, CELLS, false, OT>;
     }
 }
 
 // The step kernel for a board size L, an env kind, Discrete / multi-action, the in-place observation update, an
 // observation format (TD_OBS_F32 when no observation is written) and the opponent specialisation; NULL: none is
-// compiled.  10x10 boards hold at most 32 live enemies (one per lane), larger boards 64; other sizes take the
-// run-time-size kernels, which always write the observation in full.
+// compiled.  Boards other than 10 / 20 / 30 take the run-time-size kernels, which always write the observation in full.
 static StepKernel step_kernel(int L, int kind, bool multi, bool incremental, int obs_format, bool scripted)
 {
     if (obs_format != TD_OBS_F32) {
         if (multi) return nullptr;
         const bool bf16 = obs_format == TD_OBS_BF16;
         switch (L) {
-        case 10: return bf16 ? reduced_step_kernel<100, 1, __nv_bfloat16>(kind) : reduced_step_kernel<100, 1, uint8_t>(kind);
-        case 20: return bf16 ? reduced_step_kernel<400, 2, __nv_bfloat16>(kind) : reduced_step_kernel<400, 2, uint8_t>(kind);
-        case 30: return bf16 ? reduced_step_kernel<900, 2, __nv_bfloat16>(kind) : reduced_step_kernel<900, 2, uint8_t>(kind);
+        case 10: return bf16 ? reduced_step_kernel<100, __nv_bfloat16>(kind) : reduced_step_kernel<100, uint8_t>(kind);
+        case 20: return bf16 ? reduced_step_kernel<400, __nv_bfloat16>(kind) : reduced_step_kernel<400, uint8_t>(kind);
+        case 30: return bf16 ? reduced_step_kernel<900, __nv_bfloat16>(kind) : reduced_step_kernel<900, uint8_t>(kind);
         default: return nullptr;
         }
     }
     switch (L) {
     case 10:
-        return incremental ? f32_step_kernel<100, 32 / TD_GROUP_SMALL, TD_GROUP_SMALL, true>(kind, multi, scripted)
-                           : f32_step_kernel<100, 32 / TD_GROUP_SMALL, TD_GROUP_SMALL, false>(kind, multi, scripted);
+        return incremental ? f32_step_kernel<100, true>(kind, multi, scripted) : f32_step_kernel<100, false>(kind, multi, scripted);
     case 20:
-        return incremental ? f32_step_kernel<400, 2, 32, true>(kind, multi, scripted) : f32_step_kernel<400, 2, 32, false>(kind, multi, scripted);
+        return incremental ? f32_step_kernel<400, true>(kind, multi, scripted) : f32_step_kernel<400, false>(kind, multi, scripted);
     case 30:
-        return incremental ? f32_step_kernel<900, 2, 32, true>(kind, multi, scripted) : f32_step_kernel<900, 2, 32, false>(kind, multi, scripted);
-    default: return f32_step_kernel<0, 2, 32, false>(kind, multi, scripted);
+        return incremental ? f32_step_kernel<900, true>(kind, multi, scripted) : f32_step_kernel<900, false>(kind, multi, scripted);
+    default: return f32_step_kernel<0, false>(kind, multi, scripted);
     }
 }
 
@@ -717,10 +705,9 @@ static int launch_step(td_handle *h, const td_step_io *io, int begin, int count,
     p.io = *io;
     p.env_begin = begin;
     p.n_envs = begin + count;
-    const int wpc = step_warps_per_cta(h, incremental);
-    const int per_cta = wpc * 32 / step_group_width(h);                  // game instances per CTA
-    const int grid = (count + per_cta - 1) / per_cta, block = wpc * 32;
-    const size_t smem = wpc == kWarpsPerCta ? step_smem_bytes(h) : (size_t)per_cta * h->smem_per_warp;
+    const int wpc = step_warps_per_cta(h, incremental);                   // one env per warp
+    const int grid = (count + wpc - 1) / wpc, block = wpc * 32;
+    const size_t smem = wpc == kWarpsPerCta ? step_smem_bytes(h) : (size_t)wpc * h->smem_per_warp;
     const StepKernel kernel = step_kernel(h->L, h->kind, io->multi_action != 0, incremental,
                                           io->obs_dev ? io->obs_format : TD_OBS_F32, scripted_lv1_on_device(h, io));
     if (!kernel) return fail(h, TD_E_INVALID, "td_step: no step kernel is compiled for this configuration");
@@ -1163,8 +1150,7 @@ extern "C" int td_set_state(td_handle *h, int first_env, int n, const void *blob
     h->obs_synced = nullptr;                                    // no buffer shows the state being written
     if (!blob || first_env < 0 || n < 1 || first_env + n > h->n_envs) return fail(h, TD_E_INVALID, "td_set_state: bad range");
     const uint8_t *b = static_cast<const uint8_t *>(blob);
-    // the step kernels hold one enemy per lane on 10x10 boards (td_kernels.cuh: ecap = GW * NCHUNK = 32)
-    const int enemy_cap = h->L == 10 ? 32 : TD_CAP_ENEMIES;
+    const int enemy_cap = step_enemy_cap(h->L);
     for (int i = 0; i < n; ++i) {
         const uint8_t *rec = b + (size_t)i * h->record_bytes;
         const td_env_header *hd = reinterpret_cast<const td_env_header *>(rec);

@@ -34,19 +34,18 @@ namespace td {
 
 extern __shared__ __align__(16) uint8_t td_smem[];
 
-#ifndef TD_MIN_BLOCKS
-#define TD_MIN_BLOCKS 6
-#endif
-#ifndef TD_MIN_BLOCKS_ATK
-#define TD_MIN_BLOCKS_ATK 8      // 10x10 boards: the attacker env is latency-bound (scripted defender): 32 warps per SM at 64 registers
-#endif                           // (24 B of spills): 6 / 7 / 8 CTAs per SM = 0.2490 / 0.2440 / 0.2376 ms on B200; the other
-                                 // kinds gain nothing or lose (multi-action: +5 % at 7); its in-place-observation variant is
-                                 // best at 7 (0.2075 vs 0.2195 ms at 8)
-
-#ifndef TD_MIN_BLOCKS_DEF_SMALL
-#define TD_MIN_BLOCKS_DEF_SMALL 8   // 10x10 boards, Discrete defender env: 64 registers without spills, 8 CTAs per SM.  Lost while
-#endif                              // the step was HBM-bound (round 1); with the observation in compressible memory the SM side
-                                    // bounds it and 32 warps per SM win: def-small 0.1842 -> 0.1809 ms, in-place 0.1601 -> 0.1579 ms
+// Minimum CTAs per SM of the step kernels (__launch_bounds__), which caps their registers.  7-10 instead of 6 made
+// the rules faster but the step slower: the tighter register budget spills the uniform header scalars (DESIGN.md 7).
+constexpr int kMinBlocks = 6;
+// 10x10 boards: the attacker env is latency-bound (scripted defender): 32 warps per SM at 64 registers (24 B of
+// spills): 6 / 7 / 8 CTAs per SM = 0.2490 / 0.2440 / 0.2376 ms on B200; the other kinds gain nothing or lose
+// (multi-action: +5 % at 7).  Its in-place-observation variant is best at 7 (0.2075 vs 0.2195 ms at 8).
+constexpr int kMinBlocksAtk = 8;
+constexpr int kMinBlocksAtkInc = 7;
+// 10x10 boards, Discrete defender env: 64 registers without spills, 8 CTAs per SM.  Lost while the step was HBM-bound
+// (round 1); with the observation in compressible memory the SM side bounds it and 32 warps per SM win: def-small
+// 0.1842 -> 0.1809 ms, in-place 0.1601 -> 0.1579 ms.
+constexpr int kMinBlocksDefSmall = 8;
 
 // One env's rules for one step: load the record, apply the actions / scripted opponent, advance the board, emit
 // the per-env outputs, auto-reset.  Leaves the updated record in the slice and starts the asynchronous copy of
@@ -55,11 +54,10 @@ extern __shared__ __align__(16) uint8_t td_smem[];
 // host-resolved opponent input is set, so the other levels and the host-opponent paths are not compiled in (the
 // attacker kernel is instruction-fetch bound: 4,664 -> 4,088 SASS instructions, atk-small 0.2383 -> 0.2287 ms); OPP = -1 decides
 // all of it at run time.
-template <int KIND, bool MULTI, int NCHUNK, bool INC, int OPP, class W>
+template <int KIND, bool MULTI, bool INC, int OPP, class W>
 __device__ __forceinline__ void env_rules(const StepParams &p, const int env, W &w, uint8_t *rec, bool &dirty)
 {
     const DevConfig &cc = p.cfg;
-    constexpr int GW = W::G;
     const int lane = w.lane;
     const td_step_io &io = p.io;
     static_assert(OPP < 0 || KIND != TD_KIND_2P, "the two-player env has no scripted opponent");
@@ -80,23 +78,23 @@ __device__ __forceinline__ void env_rules(const StepParams &p, const int env, W 
         // where summon_cluster turns it into the RealAction in place (no registers held across the step)
         const long long *src = reinterpret_cast<const long long *>(io.atk_action_dev) + (size_t)env * TD_ROADS * TD_CLUSTER;
         if ((reinterpret_cast<uintptr_t>(io.atk_action_dev) & 15) == 0) {
-            async_copy16(w.act_stage(), src, TD_ROADS * TD_CLUSTER / 2, lane, GW);
+            async_copy16(w.act_stage(), src, TD_ROADS * TD_CLUSTER / 2, lane);
             asm volatile("cp.async.commit_group;" ::: "memory");
         } else {
-            for (int q = lane; q < TD_ROADS * TD_CLUSTER; q += GW) w.act_stage()[q] = src[q];
+            for (int q = lane; q < TD_ROADS * TD_CLUSTER; q += kLanes) w.act_stage()[q] = src[q];
         }
     }
     if (KIND == TD_KIND_DEF && OPP < 0 && io.opponent_dev != nullptr) in_opp = io.opponent_dev[env];
-    w.ecap = GW * NCHUNK;
+    w.ecap = step_enemy_cap(W::kL);
     asm volatile("cp.async.wait_group 0;" ::: "memory");
-    gsync(w);
+    __syncwarp();
     finish_env_load(w, p, rec, device_opponent ? p.mt + (size_t)env * kMtWords : nullptr);
     if (INC) {
         // remember where towers and enemies stand in the observation the caller's buffer still holds
         uint32_t *old = w.old_lists();
         if (lane == 0) { old[0] = (uint32_t)w.nt; old[1] = (uint32_t)w.ne; }
-        for (int t = lane; t < w.nt; t += GW) old[4 + t] = w.tw()[t].loc | ((uint32_t)w.tw()[t].type_lv << 16);
-        for (int e = lane; e < w.ne; e += GW) old[4 + TD_CAP_TOWERS + e] = w.en()[e].loc | ((uint32_t)(w.en()[e].type_lv & 3) << 16);
+        for (int t = lane; t < w.nt; t += kLanes) old[4 + t] = w.tw()[t].loc | ((uint32_t)w.tw()[t].type_lv << 16);
+        for (int e = lane; e < w.ne; e += kLanes) old[4 + TD_CAP_TOWERS + e] = w.en()[e].loc | ((uint32_t)(w.en()[e].type_lv & 3) << 16);
     }
 
     // cooldowns (TDDefense.py:38-39)
@@ -127,7 +125,7 @@ __device__ __forceinline__ void env_rules(const StepParams &p, const int env, W 
                 int code = 0;
                 bool skip = false;
                 if (!(KIND == TD_KIND_2P && MULTI))
-                    skip = gall(w, lane >= TD_CLUSTER || cur == TD_NTYPES);           // TDAttack.py:39-41
+                    skip = __all_sync(kFull, lane >= TD_CLUSTER || cur == TD_NTYPES);           // TDAttack.py:39-41
                 if (!skip) {
                     const long long before = cur;
                     const bool res = summon_cluster(w, i, cur, 0);
@@ -175,11 +173,11 @@ __device__ __forceinline__ void env_rules(const StepParams &p, const int env, W 
             w.cache_raw = true;
             w.ck = 0;
             w.cn = min(w.rng_words(), max(kMtWords - w.mt_pos, 0));
-            constexpr int kRefill = (W::kRngWords + GW - 1) / GW;
+            constexpr int kRefill = (W::kRngWords + kLanes - 1) / kLanes;
             const unsigned dst = (unsigned)__cvta_generic_to_shared(w.rng_cache());
 #pragma unroll
             for (int q = 0; q < kRefill; ++q) {
-                const int k = lane + GW * q;
+                const int k = lane + kLanes * q;
                 if (k < w.cn)
                     asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst + 4u * k), "l"(w.mt + w.mt_pos + k) : "memory");
                 else if (k < W::kRngWords)
@@ -189,10 +187,10 @@ __device__ __forceinline__ void env_rules(const StepParams &p, const int env, W 
         asm volatile("cp.async.commit_group;" ::: "memory");
     };
     if (INC) refill();          // in-place observation kernels write the record back first (see td_step_kernel)
-    gsync(w);
+    __syncwarp();
 
     int kills, leaks;
-    double reward = board_step<NCHUNK>(w, kills, leaks);
+    double reward = board_step(w, kills, leaks);
     if (KIND == TD_KIND_ATK) reward = -reward;
 
     const bool has_base = cc.base_LP >= 0;
@@ -239,7 +237,7 @@ __device__ __forceinline__ void env_rules(const StepParams &p, const int env, W 
         if (w.flags) p.stats[env].flags |= (uint32_t)w.flags;
     }
     if (KIND != TD_KIND_DEF && io.real_atk_dev) {
-        for (int q = lane; q < TD_ROADS * TD_CLUSTER; q += GW)
+        for (int q = lane; q < TD_ROADS * TD_CLUSTER; q += kLanes)
             io.real_atk_dev[(size_t)env * TD_ROADS * TD_CLUSTER + q] = w.act_stage()[q];
     }
     if (io.packed_out_dev != nullptr) {
@@ -262,7 +260,7 @@ __device__ __forceinline__ void env_rules(const StepParams &p, const int env, W 
         if (lane < kStride / 16) po[lane] = v;
     }
     (void)def_ok;
-    gsync(w);
+    __syncwarp();
 
     if (__builtin_expect(done && io.auto_reset, 0)) {
         int next = (w.hdr()->map_id + p.map_stride) % p.n_maps;
@@ -275,21 +273,20 @@ __device__ __forceinline__ void env_rules(const StepParams &p, const int env, W 
 
 // INC: the observation is an in-place update of the previous one (td_step_io.obs_incremental, vouched for by the
 // engine); a separate instantiation, so that the full-write kernels carry none of its code.
-template <int KIND, bool MULTI, int CELLS, int NCHUNK, int GW, bool INC, class OT = float, int OPP = -1>
-__global__ void __launch_bounds__(kWarpsPerCta * 32, (KIND == TD_KIND_ATK && CELLS == 100) ? (INC ? 7 : TD_MIN_BLOCKS_ATK)
-                                                     : (KIND == TD_KIND_DEF && !MULTI && CELLS == 100) ? TD_MIN_BLOCKS_DEF_SMALL : TD_MIN_BLOCKS)
+template <int KIND, bool MULTI, int CELLS, bool INC, class OT = float, int OPP = -1>
+__global__ void __launch_bounds__(kWarpsPerCta * 32, (KIND == TD_KIND_ATK && CELLS == 100) ? (INC ? kMinBlocksAtkInc : kMinBlocksAtk)
+                                                     : (KIND == TD_KIND_DEF && !MULTI && CELLS == 100) ? kMinBlocksDefSmall : kMinBlocks)
 td_step_kernel(const __grid_constant__ StepParams p)
 {
-    // one group of GW lanes per game instance (GW = 16: two instances share a warp)
-    const int group = threadIdx.x / GW;
-    const int env = p.env_begin + blockIdx.x * (blockDim.x / GW) + group;      // any CTA size up to kWarpsPerCta warps
+    const int warp = threadIdx.x / 32;
+    const int env = p.env_begin + blockIdx.x * (blockDim.x / 32) + warp;      // any CTA size up to kWarpsPerCta warps
     if (env >= p.n_envs) return;
     constexpr int RC = KIND == TD_KIND_ATK ? kRngCacheAtk : kRngCacheDef;
-    Ctx<CELLS, GW, RC> w;
-    ctx_bind(w, td_smem + (size_t)group * p.smem_per_warp, p);               // [record | scratch] per instance
+    Ctx<CELLS, RC> w;
+    ctx_bind(w, td_smem + (size_t)warp * p.smem_per_warp, p);               // [record | scratch] per warp
     uint8_t *rec = p.records + (size_t)env * w.record_bytes();
     bool dirty = false;
-    env_rules<KIND, MULTI, NCHUNK, INC, OPP>(p, env, w, rec, dirty);
+    env_rules<KIND, MULTI, INC, OPP>(p, env, w, rec, dirty);
     // The header scalars go back to the slice before the observation is written: their registers are free
     // during the store phase (a spilled one cost a local-memory reload behind 18 KB of stores: 8 % of the step).
     push_header(w);
@@ -298,7 +295,7 @@ td_step_kernel(const __grid_constant__ StepParams p)
     // kernels keep the record for last: 0.2175 vs 0.2206 ms on def-small.
     if (INC) {
         asm volatile("cp.async.wait_group 0;" ::: "memory");
-        if (w.cache_raw) { gsync(w); temper_cache(w); }
+        if (w.cache_raw) { __syncwarp(); temper_cache(w); }
         store_env<true>(w, p, rec, dirty, false);
     }
     if (p.io.obs_dev) {
@@ -306,7 +303,7 @@ td_step_kernel(const __grid_constant__ StepParams p)
         if constexpr (INC && CELLS > 0) {
             obs_prepare(w);
             if (!w.static_dirty && (reinterpret_cast<uintptr_t>(o) & 15) == 0) obs_dense_incremental(w, o);
-            else obs_dense<GW>(w, o, w.lane);              // envs restarted inside this step get all 45 planes
+            else obs_dense(w, o);                          // envs restarted inside this step get all 45 planes
             obs_sparse(w, o);
         } else {
             write_obs(w, o);
@@ -314,7 +311,7 @@ td_step_kernel(const __grid_constant__ StepParams p)
     }
     if (!INC) {
         asm volatile("cp.async.wait_group 0;" ::: "memory");      // the next steps' generator words are in the slice
-        if (w.cache_raw) { gsync(w); temper_cache(w); }
+        if (w.cache_raw) { __syncwarp(); temper_cache(w); }
         store_env<(KIND == TD_KIND_ATK)>(w, p, rec, dirty, false);
     }
 }
@@ -327,17 +324,17 @@ td_reset_kernel(const __grid_constant__ StepParams p, const uint8_t *mask, const
     const int env = blockIdx.x * kWarpsPerCta + warp;
     if (env >= p.n_envs) return;
     if (mask && !mask[env]) return;
-    Ctx<0, 32> w;
+    Ctx<0> w;
     ctx_bind(w, td_smem + (size_t)warp * p.smem_per_warp, p);
     uint8_t *rec = p.records + (size_t)env * p.record_bytes;
     if (w.lane < (w.hdr_bytes() >> 4)) reinterpret_cast<int4 *>(w.hdr())[w.lane] = reinterpret_cast<const int4 *>(rec)[w.lane];
-    gsync(w);
+    __syncwarp();
     pull_header(w);
     int id = map_ids ? map_ids[env] : env % p.n_maps;
     id = ((id % p.n_maps) + p.n_maps) % p.n_maps;
     reset_env(w, p, id, true);
     if (obs) write_obs(w, obs + (size_t)env * TD_NCHANNELS * w.ncells());
-    gsync(w);
+    __syncwarp();
     store_env(w, p, rec, true);
 }
 
@@ -347,7 +344,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) td_observe_kernel(const __g
     const int warp = threadIdx.x >> 5;
     const int env = blockIdx.x * kWarpsPerCta + warp;
     if (env >= p.n_envs) return;
-    Ctx<CELLS, 32> w;
+    Ctx<CELLS> w;
     ctx_bind(w, td_smem + (size_t)warp * p.smem_per_warp, p);
     load_env(w, p, p.records + (size_t)env * p.record_bytes);
     write_obs(w, obs + (size_t)env * TD_NCHANNELS * w.ncells());

@@ -10,37 +10,37 @@ namespace td {
 
 // Regenerate the 624 words in place.  mt[k] = mt[(k+397)%624] ^ f(mt[k], mt[k+1]); chunks of 32 words in
 // ascending order keep every operand in the state (old / new) the sequential algorithm sees.
-__device__ __noinline__ void mt_twist(uint32_t *mt, int lane, int stride, unsigned gmask)
+__device__ __noinline__ void mt_twist(uint32_t *mt, int lane)
 {
 #pragma unroll 1
-    for (int base = 0; base < kMtWords; base += stride) {
+    for (int base = 0; base < kMtWords; base += kLanes) {
         const int k = base + lane;
         uint32_t v = 0;
         if (k < kMtWords - 1) {
             uint32_t y = (mt[k] & 0x80000000u) | (mt[k + 1] & 0x7fffffffu);
             v = mt[k < 227 ? k + 397 : k - 227] ^ (y >> 1) ^ ((y & 1u) ? 0x9908b0dfu : 0u);
         }
-        __syncwarp(gmask);
+        __syncwarp();
         if (k < kMtWords - 1) mt[k] = v;
-        __syncwarp(gmask);
+        __syncwarp();
     }
     if (lane == 0) {
         uint32_t y = (mt[623] & 0x80000000u) | (mt[0] & 0x7fffffffu);
         mt[623] = mt[396] ^ (y >> 1) ^ ((y & 1u) ? 0x9908b0dfu : 0u);
     }
-    __syncwarp(gmask);
+    __syncwarp();
 }
 
 // The same through shared memory: the 20 dependent chunks of the regeneration cost one HBM round trip each when
 // run on the state in place (40 us per twist under load); staged, the state travels once in and once out.
-// gmt is 16-byte aligned (624 words per env), smt is a 2496-byte staging area in the group's slice.
-__device__ __noinline__ void mt_twist_staged(uint32_t *gmt, uint32_t *smt, int lane, int stride, unsigned gmask)
+// gmt is 16-byte aligned (624 words per env), smt is a 2496-byte staging area in the warp's slice.
+__device__ __noinline__ void mt_twist_staged(uint32_t *gmt, uint32_t *smt, int lane)
 {
-    for (int q = lane; q < kMtWords / 4; q += stride) reinterpret_cast<int4 *>(smt)[q] = reinterpret_cast<const int4 *>(gmt)[q];
-    __syncwarp(gmask);
-    mt_twist(smt, lane, stride, gmask);
-    for (int q = lane; q < kMtWords / 4; q += stride) reinterpret_cast<int4 *>(gmt)[q] = reinterpret_cast<const int4 *>(smt)[q];
-    __syncwarp(gmask);
+    for (int q = lane; q < kMtWords / 4; q += kLanes) reinterpret_cast<int4 *>(smt)[q] = reinterpret_cast<const int4 *>(gmt)[q];
+    __syncwarp();
+    mt_twist(smt, lane);
+    for (int q = lane; q < kMtWords / 4; q += kLanes) reinterpret_cast<int4 *>(gmt)[q] = reinterpret_cast<const int4 *>(smt)[q];
+    __syncwarp();
 }
 
 __device__ __forceinline__ uint32_t mt_temper(uint32_t y)
@@ -58,14 +58,13 @@ __device__ __forceinline__ uint32_t mt_temper(uint32_t y)
 // back).  Only when a step needs more words than the cache holds (the scripted defender's shuffle, a few percent
 // of its steps) the out-of-line refill fetches them from the generator state in HBM, twisting it when exhausted.
 struct MtRefill { int cn, mt_pos; };
-__device__ __noinline__ MtRefill mt_refill(uint32_t *cache, uint32_t *mt, uint32_t *stage, int lane, int G, unsigned gmask,
-                                           int mt_pos, int words)
+__device__ __noinline__ MtRefill mt_refill(uint32_t *cache, uint32_t *mt, uint32_t *stage, int lane, int mt_pos, int words)
 {
-    if (mt_pos >= kMtWords) { mt_twist_staged(mt, stage, lane, G, gmask); mt_pos = 0; }
+    if (mt_pos >= kMtWords) { mt_twist_staged(mt, stage, lane); mt_pos = 0; }
     const int n = min(words, kMtWords - mt_pos);
-    __syncwarp(gmask);                                  // every earlier read of the cache is done
-    for (int q = lane; q < n; q += G) cache[q] = mt_temper(mt[mt_pos + q]);
-    __syncwarp(gmask);
+    __syncwarp();                                       // every earlier read of the cache is done
+    for (int q = lane; q < n; q += kLanes) cache[q] = mt_temper(mt[mt_pos + q]);
+    __syncwarp();
     MtRefill r;
     r.cn = n;
     r.mt_pos = mt_pos;
@@ -75,8 +74,8 @@ __device__ __noinline__ MtRefill mt_refill(uint32_t *cache, uint32_t *mt, uint32
 template <class W>
 __device__ __forceinline__ void mt_more_words(W &w)
 {
-    const MtRefill r = mt_refill(const_cast<uint32_t *>(w.rng_cache()), w.mt, w.twist_stage(), w.lane, W::G, w.gmask,
-                                 w.mt_pos, w.rng_words());
+    const MtRefill r = mt_refill(const_cast<uint32_t *>(w.rng_cache()), w.mt, w.twist_stage(), w.lane, w.mt_pos,
+                                 w.rng_words());
     w.cn = r.cn;
     w.mt_pos = r.mt_pos;
     w.ck = 0;
@@ -88,17 +87,17 @@ template <class W>
 __device__ __forceinline__ void temper_cache(W &w)
 {
     uint32_t *cache = const_cast<uint32_t *>(w.rng_cache());
-    constexpr int kIters = W::kRngWords > 0 ? (W::kRngWords + W::G - 1) / W::G : 0;
+    constexpr int kIters = W::kRngWords > 0 ? (W::kRngWords + kLanes - 1) / kLanes : 0;
     if (kIters > 0) {
 #pragma unroll
         for (int it = 0; it < kIters; ++it) {
-            const int q = w.lane + W::G * it;
+            const int q = w.lane + kLanes * it;
             if (q < w.cn) cache[q] = mt_temper(cache[q]);
         }
     } else {
-        for (int q = w.lane; q < w.cn; q += W::G) cache[q] = mt_temper(cache[q]);
+        for (int q = w.lane; q < w.cn; q += kLanes) cache[q] = mt_temper(cache[q]);
     }
-    gsync(w);
+    __syncwarp();
 }
 
 template <class W>
@@ -125,7 +124,7 @@ __device__ __forceinline__ int py_randbelow(W &w, int n)
 // random.shuffle(list) (for i in reversed(range(1, n)): j = randbelow(i + 1); swap) on a uint16 list in shared
 // memory.  The draws are serial by definition (rejections shift every later draw), so one lane runs the whole
 // loop alone, straight over the tempered word cache -- a fifth of the instructions of the same loop with a
-// group-wide draw per element.
+// warp-wide draw per element.
 template <class W>
 __device__ __forceinline__ void py_shuffle_u16(W &w, uint16_t *list, int n)
 {
@@ -147,11 +146,11 @@ __device__ __forceinline__ void py_shuffle_u16(W &w, uint16_t *list, int n)
                 }
             }
         }
-        k = gshfl(w, k, 0);
-        i = gshfl(w, i, 0);
+        k = __shfl_sync(kFull, k, 0);
+        i = __shfl_sync(kFull, i, 0);
         w.mt_pos += k - w.ck;
         w.ck = k;
-        gsync(w);
+        __syncwarp();
     }
 }
 

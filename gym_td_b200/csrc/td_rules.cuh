@@ -11,24 +11,23 @@ namespace td {
 
 // map[6] += delta on the Manhattan diamond around `loc` (TDBoard.py:239-245, 281-287).  Out of line: it is
 // reached from several build / destruct sites and only on the rare successful operation.
-__device__ __noinline__ void diamond_add_cells(uint8_t *map6, int loc, int delta, int L, int D, int lane, int stride,
-                                               unsigned gmask)
+__device__ __noinline__ void diamond_add_cells(uint8_t *map6, int loc, int delta, int L, int D, int lane)
 {
     const int WD = 2 * D + 1;
     const int r0 = loc / L, c0 = loc - r0 * L;
-    for (int k = lane; k < WD * WD; k += stride) {
+    for (int k = lane; k < WD * WD; k += kLanes) {
         int i = k / WD - D, j = k % WD - D;
         int r = r0 + i, c = c0 + j;
         if (abs(i) + abs(j) <= D && r >= 0 && r < L && c >= 0 && c < L)
             map6[r * L + c] = (uint8_t)(map6[r * L + c] + delta);
     }
-    __syncwarp(gmask);
+    __syncwarp();
 }
 
 template <class W>
 __device__ __forceinline__ void diamond_add(W &w, int loc, int delta)
 {
-    diamond_add_cells(w.map6(), loc, delta, w.L(), w.pp->cfg.tower_distance, w.lane, W::G, w.gmask);
+    diamond_add_cells(w.map6(), loc, delta, w.L(), w.pp->cfg.tower_distance, w.lane);
 }
 
 template <class W>
@@ -58,9 +57,9 @@ template <class W>
 __device__ __forceinline__ int find_tower(const W &w, int loc)
 {
     int idx = -1;
-    for (int base = 0; base < w.nt; base += W::G) {
+    for (int base = 0; base < w.nt; base += kLanes) {
         const int t = base + w.lane;
-        const unsigned b = gballot(w, t < w.nt && w.tw()[t].loc == loc);
+        const unsigned b = __ballot_sync(kFull, t < w.nt && w.tw()[t].loc == loc);
         if (b && idx < 0) idx = base + __ffs(b) - 1;
     }
     return idx;
@@ -76,9 +75,9 @@ __device__ __forceinline__ bool tower_lvup(W &w, int loc)                       
     if (lv >= TD_NLV - 1) { w.fail = TD_FC_LV_MAX; return false; }
     const double cost = cc.tower_cost[ty][lv + 1];
     if (w.cost_def < cost) { w.fail = TD_FC_COST_SHORTAGE; return false; }
-    gsync(w);
+    __syncwarp();
     if (w.lane == 0) w.tw()[idx].type_lv = (uint8_t)(ty | ((lv + 1) << 2));
-    gsync(w);
+    __syncwarp();
     w.cost_def = __dsub_rn(w.cost_def, cost);
     w.fail = TD_FC_SUCCESS;
     return true;
@@ -94,20 +93,20 @@ __device__ __forceinline__ bool tower_destruct(W &w, int loc, bool &map6_dirty) 
     double c = __dadd_rn(w.cost_def, __dmul_rn(cc.tower_refund[tl & 3][tl >> 2], cc.destruct_return));
     w.cost_def = cc.max_cost < c ? cc.max_cost : c;
     // remove from the list, keeping the order of the rest
-    constexpr int kPasses = TD_CAP_TOWERS / W::G;
+    constexpr int kPasses = TD_CAP_TOWERS / kLanes;
     td_tower_rec mine[kPasses];
 #pragma unroll
     for (int q = 0; q < kPasses; ++q) {
-        const int t = w.lane + W::G * q;
+        const int t = w.lane + kLanes * q;
         if (t > idx && t < w.nt) mine[q] = w.tw()[t];
     }
-    gsync(w);
+    __syncwarp();
 #pragma unroll
     for (int q = 0; q < kPasses; ++q) {
-        const int t = w.lane + W::G * q;
+        const int t = w.lane + kLanes * q;
         if (t > idx && t < w.nt) w.tw()[t - 1] = mine[q];
     }
-    gsync(w);
+    __syncwarp();
     w.nt -= 1;
     diamond_add(w, loc, -1);
     map6_dirty = true;
@@ -147,11 +146,11 @@ __device__ __forceinline__ void decode_multi(W &w, const long long *act, long lo
     const int cells = w.ncells();
     uint8_t *tower_at = w.scratch();      // cells bytes: 1 where a tower stands (scratch >= cells_pad here)
     const bool enabled = w.def_cd == 0;
-    for (int q = w.lane; q < (w.cells_pad() >> 2); q += W::G) reinterpret_cast<uint32_t *>(tower_at)[q] = 0u;
-    gsync(w);
-    for (int t = w.lane; t < w.nt; t += W::G) tower_at[w.tw()[t].loc] = 1;
-    gsync(w);
-    for (int base = 0; base < cells; base += W::G) {
+    for (int q = w.lane; q < (w.cells_pad() >> 2); q += kLanes) reinterpret_cast<uint32_t *>(tower_at)[q] = 0u;
+    __syncwarp();
+    for (int t = w.lane; t < w.nt; t += kLanes) tower_at[w.tw()[t].loc] = 1;
+    __syncwarp();
+    for (int base = 0; base < cells; base += kLanes) {
         const int cell = base + w.lane;
         unsigned flags = 0;          // bit ch set when action[ch][cell] == 1
         if (cell < cells) {
@@ -163,7 +162,7 @@ __device__ __forceinline__ void decode_multi(W &w, const long long *act, long lo
         }
         unsigned done_mask = 0;      // successes of this lane's cell
         if (enabled) {
-            unsigned pending = gballot(w, flags != 0);
+            unsigned pending = __ballot_sync(kFull, flags != 0);
             while (pending) {
                 // screen with the current state
                 bool can = false;
@@ -176,16 +175,16 @@ __device__ __forceinline__ void decode_multi(W &w, const long long *act, long lo
                     }
                     // a flagged build on a free cell can create the tower that a flagged LvUp/destruct then hits
                 }
-                unsigned cand = gballot(w, can) & pending;
+                unsigned cand = __ballot_sync(kFull, can) & pending;
                 if (!cand) break;
                 int src = __ffs(cand) - 1;
-                unsigned f = gshfl(w, flags, src);
+                unsigned f = __shfl_sync(kFull, flags, src);
                 int loc = base + src;
                 unsigned ok = 0;
                 for (int t = 0; t < TD_NTYPES; ++t)
-                    if ((f >> t) & 1u) if (tower_build(w, t, loc, dirty)) { ok |= 1u << t; if (w.lane == 0) tower_at[loc] = 1; gsync(w); }
+                    if ((f >> t) & 1u) if (tower_build(w, t, loc, dirty)) { ok |= 1u << t; if (w.lane == 0) tower_at[loc] = 1; __syncwarp(); }
                 if ((f >> 4) & 1u) if (tower_lvup(w, loc)) ok |= 1u << 4;
-                if ((f >> 5) & 1u) if (tower_destruct(w, loc, dirty)) { ok |= 1u << 5; if (w.lane == 0) tower_at[loc] = 0; gsync(w); }
+                if ((f >> 5) & 1u) if (tower_destruct(w, loc, dirty)) { ok |= 1u << 5; if (w.lane == 0) tower_at[loc] = 0; __syncwarp(); }
                 if (ok) w.def_cd = cc.def_interval;
                 if (w.lane == src) done_mask = ok;
                 // cells up to and including src are finished
@@ -197,7 +196,7 @@ __device__ __forceinline__ void decode_multi(W &w, const long long *act, long lo
             for (int ch = 0; ch < 6; ++ch) __stcs(real + (size_t)ch * cells + cell, (long long)((done_mask >> ch) & 1u));
         }
     }
-    gsync(w);
+    __syncwarp();
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -230,8 +229,8 @@ __device__ __forceinline__ bool summon_cluster(W &w, int road, long long &mine, 
     const int start = w.mh()->start[road];
     const int lv = w.steps >= cc.upgrade_step ? 1 : 0;      // progress >= enemy_upgrade_at
     const int tv = (mine < 0 || mine >= TD_NTYPES) ? TD_NTYPES : (int)mine;     // 4 == enemy_types: empty slot
-    const unsigned b0 = gballot(w, tv & 1) >> lane_base, b1 = gballot(w, tv & 2) >> lane_base,
-                   b2 = gballot(w, tv & 4) >> lane_base;
+    const unsigned b0 = __ballot_sync(kFull, tv & 1) >> lane_base, b1 = __ballot_sync(kFull, tv & 2) >> lane_base,
+                   b2 = __ballot_sync(kFull, tv & 4) >> lane_base;
     unsigned todo = ~b2 & 0xffu;                     // slots holding a real type (0..3)
     const bool tried = todo != 0;
     unsigned ok = 0, poor = 0;
@@ -261,7 +260,7 @@ __device__ __forceinline__ bool summon_cluster(W &w, int road, long long &mine, 
         }
     }
     w.ne += n;
-    gsync(w);
+    __syncwarp();
     if (ok == 0 && tried) { w.fail = TD_FC_COST_SHORTAGE; return false; }
     w.fail = TD_FC_SUCCESS;
     return true;
@@ -295,7 +294,7 @@ __device__ __forceinline__ void summon_uniform(W &w, int t, int road)
         e.slowdown = 0;
     }
     w.ne += n;
-    gsync(w);
+    __syncwarp();
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -344,11 +343,11 @@ __device__ __forceinline__ void opponent_tower(W &w, int difficulty, bool &dirty
             // TDGymBasic.py:216-240: counter the enemy type drawn in proportion to the live enemies
             if (w.ne == 0) return;
             int cnt[TD_NTYPES] = {0, 0, 0, 0};
-            for (int base = 0; base < w.ne; base += W::G) {
+            for (int base = 0; base < w.ne; base += kLanes) {
                 const int e = base + w.lane;
                 const int ty = e < w.ne ? (w.en()[e].type_lv & 3) : -1;
 #pragma unroll
-                for (int q = 0; q < TD_NTYPES; ++q) cnt[q] += __popc(gballot(w, ty == q));
+                for (int q = 0; q < TD_NTYPES; ++q) cnt[q] += __popc(__ballot_sync(kFull, ty == q));
             }
             double p = py_random(w);
             int pick = -1, last = 0;
@@ -367,15 +366,15 @@ __device__ __forceinline__ void opponent_tower(W &w, int difficulty, bool &dirty
         // road cells in row-major order
         uint16_t *list = reinterpret_cast<uint16_t *>(w.scratch());
         int n = 0;
-        for (int base = 0; base < w.ncells(); base += W::G) {
+        for (int base = 0; base < w.ncells(); base += kLanes) {
             int c = base + w.lane;
             bool on = c < w.ncells() && (w.cells()[c] & 1);
-            unsigned b = gballot(w, on);
+            unsigned b = __ballot_sync(kFull, on);
             TD_CHECK(w, 2 * (n + __popc(b)) <= max(768, w.cells_pad()));
             if (on) list[n + __popc(b & ((1u << w.lane) - 1u))] = (uint16_t)c;
             n += __popc(b);
         }
-        gsync(w);
+        __syncwarp();
         py_shuffle_u16(w, list, n);
         if (difficulty != 2) t = py_randbelow(w, TD_NTYPES);
         for (int k = 0; k < n; ++k) {
@@ -405,9 +404,10 @@ struct EnemyRegs {
     bool valid;
 };
 
-template <int NCHUNK, class W>
+template <class W>
 __device__ __forceinline__ double board_step(W &w, int &kills_out, int &leaks_out)
 {
+    constexpr int NCHUNK = step_enemy_cap(W::kL) / kLanes;     // enemies per lane
     const DevConfig &cc = w.pp->cfg;
     const int L = w.L(), lane = w.lane;
     double reward = __dadd_rn(0.0, cc.reward_time);
@@ -423,7 +423,7 @@ __device__ __forceinline__ double board_step(W &w, int &kills_out, int &leaks_ou
     bool unsorted = false;
 #pragma unroll
     for (int k = 0; k < NCHUNK; ++k) {
-        int e = lane + W::G * k;
+        int e = lane + kLanes * k;
         E[k].valid = e < ne;
         if (E[k].valid) {
             const td_enemy_rec &x = w.en()[e];
@@ -431,14 +431,14 @@ __device__ __forceinline__ double board_step(W &w, int &kills_out, int &leaks_ou
             keys[e] = __dsub_rn((double)w.dist()[E[k].loc], E[k].margin);
         }
     }
-    gsync(w);
+    __syncwarp();
 #pragma unroll
     for (int k = 0; k < NCHUNK; ++k) {
-        int e = lane + W::G * k;
+        int e = lane + kLanes * k;
         bool inv = E[k].valid && e > 0 && keys[e - 1] > keys[e];
         unsorted = unsorted || inv;
     }
-    unsorted = gany(w, unsorted);
+    unsorted = __any_sync(kFull, unsorted);
     if (unsorted) {
         // stable rank = #(key smaller) + #(equal key, earlier position)
         int rank[NCHUNK];
@@ -448,11 +448,11 @@ __device__ __forceinline__ double board_step(W &w, int &kills_out, int &leaks_ou
             double kj = keys[j];
 #pragma unroll
             for (int k = 0; k < NCHUNK; ++k) {
-                int e = lane + W::G * k;
+                int e = lane + kLanes * k;
                 if (E[k].valid) { double ke = keys[e]; rank[k] += (kj < ke || (kj == ke && j < e)) ? 1 : 0; }
             }
         }
-        gsync(w);
+        __syncwarp();
 #pragma unroll
         for (int k = 0; k < NCHUNK; ++k)
             if (E[k].valid) {
@@ -461,10 +461,10 @@ __device__ __forceinline__ double board_step(W &w, int &kills_out, int &leaks_ou
                 x.LP = E[k].LP; x.margin = E[k].margin; x.loc = (uint16_t)E[k].loc; x.type_lv = (uint8_t)E[k].tl;
                 x.slowdown = (uint8_t)E[k].slow;
             }
-        gsync(w);
+        __syncwarp();
 #pragma unroll
         for (int k = 0; k < NCHUNK; ++k) {
-            int e = lane + W::G * k;
+            int e = lane + kLanes * k;
             if (E[k].valid) {
                 const td_enemy_rec &x = w.en()[e];
                 E[k].LP = x.LP; E[k].margin = x.margin; E[k].loc = x.loc; E[k].tl = x.type_lv; E[k].slow = x.slowdown;
@@ -473,19 +473,19 @@ __device__ __forceinline__ double board_step(W &w, int &kills_out, int &leaks_ou
     }
 #pragma unroll
     for (int k = 0; k < NCHUNK; ++k) {
-        int e = lane + W::G * k;
+        int e = lane + kLanes * k;
         if (E[k].valid) {
             E[k].r = E[k].loc / L; E[k].c = E[k].loc - E[k].r * L;
             erow[e] = (uint8_t)E[k].r; ecol[e] = (uint8_t)E[k].c;
         }
     }
-    gsync(w);
+    __syncwarp();
 
     // ---- towers choose targets: first enemy in list order within Chebyshev range, corpses included
     //      (TDBoard.py:306-312, TDElements.py:72-132).  Positions do not change inside the tower loop, so
     //      every tower's choice is independent: lane = tower.
     uint8_t *fire = w.scratch() + 640, *vict = w.scratch() + 672;     // [32] each
-    for (int tt = lane; tt < nt; tt += W::G) {
+    for (int tt = lane; tt < nt; tt += kLanes) {
         td_tower_rec &T = w.tw()[tt];
         const int ty = T.type_lv & 3, lv = T.type_lv >> 2;
         double cd = __dsub_rn(T.cd, 1.0);
@@ -517,7 +517,7 @@ __device__ __forceinline__ double board_step(W &w, int &kills_out, int &leaks_ou
         fire[tt] = (uint8_t)(target < 0 ? 0xff : target);
         vict[tt] = (uint8_t)(victim < 0 ? 0xff : victim);
     }
-    gsync(w);
+    __syncwarp();
 
     // ---- damage in tower order: lane = enemy (TDElements.py:19-28)
     bool hit[NCHUNK];
@@ -538,7 +538,7 @@ __device__ __forceinline__ double board_step(W &w, int &kills_out, int &leaks_ou
             const int fr = erow[f], fc = ecol[f], v = vict[t];
 #pragma unroll
             for (int k = 0; k < NCHUNK; ++k) {
-                int e = lane + W::G * k;
+                int e = lane + kLanes * k;
                 bool h;
                 if (ty == 2) h = E[k].valid && max(abs(E[k].r - fr), abs(E[k].c - fc)) <= sp;
                 else if (ty == 3) h = E[k].valid && e == v;
@@ -562,7 +562,7 @@ __device__ __forceinline__ double board_step(W &w, int &kills_out, int &leaks_ou
     const int end = w.mh()->end;
     int newidx[NCHUNK];
     bool keep[NCHUNK];
-    gsync(w);
+    __syncwarp();
 #pragma unroll
     for (int k = 0; k < NCHUNK; ++k) {
         bool killed = E[k].valid && hit[k] && !(E[k].LP > 0.0);
@@ -580,7 +580,7 @@ __device__ __forceinline__ double board_step(W &w, int &kills_out, int &leaks_ou
             }
         }
         keep[k] = E[k].valid && !killed && !leaked;
-        unsigned bk = gballot(w, killed), bl = gballot(w, leaked), bs = gballot(w, keep[k]);
+        unsigned bk = __ballot_sync(kFull, killed), bl = __ballot_sync(kFull, leaked), bs = __ballot_sync(kFull, keep[k]);
         kills += __popc(bk);
         leaks += __popc(bl);
         newidx[k] = kept_before + __popc(bs & ((1u << lane) - 1u));
@@ -595,7 +595,7 @@ __device__ __forceinline__ double board_step(W &w, int &kills_out, int &leaks_ou
             x.slowdown = (uint8_t)E[k].slow;
         }
     w.ne = kept_before;
-    gsync(w);
+    __syncwarp();
 
     reward = __dadd_rn(reward, __dmul_rn(cc.reward_kill, (double)kills));
     const bool has_base = cc.base_LP >= 0;
