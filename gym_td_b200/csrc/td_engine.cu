@@ -361,6 +361,19 @@ static const void *observe_kernel(int L, int obs_format)
     }
 }
 
+// The action-mask kernel for a board size: specialised on 10 / 20 / 30, the run-time-size kernel otherwise.
+static const void *action_mask_kernel(int L)
+{
+    switch (L) {
+    case 10: return (const void *)td_action_mask_kernel<100>;
+    case 20: return (const void *)td_action_mask_kernel<400>;
+    case 30: return (const void *)td_action_mask_kernel<900>;
+    default: return (const void *)td_action_mask_kernel<0>;
+    }
+}
+
+static size_t mask_smem_of(const td_handle *h) { return (size_t)kWarpsPerCta * mask_smem_per_warp(h->cells_pad); }
+
 template <typename K> static cudaError_t allow_smem(K kernel, size_t bytes)
 {
     if (bytes <= 48 * 1024) return cudaSuccess;
@@ -412,6 +425,7 @@ extern "C" int td_create(const td_config *cfg, int env_kind, int map_size, int n
     // pick for its board size and env kind
     auto allow = [&](auto kernel, size_t bytes) { if (kernel && e == cudaSuccess) e = allow_smem(kernel, bytes); };
     allow(td_reset_kernel, smem);
+    allow(action_mask_kernel(h->L), mask_smem_of(h));
     for (int fmt : {TD_OBS_F32, TD_OBS_BF16, TD_OBS_U8}) {
         allow(observe_kernel(h->L, fmt), smem);
         for (bool multi : {false, true})
@@ -784,6 +798,34 @@ extern "C" int td_observe_as(td_handle *h, int obs_format, void *obs_dev, void *
     if (h->n_maps < 1) return fail(h, TD_E_STATE, "td_observe_as: upload maps and reset first");
     TD_CUDA(h, cudaSetDevice(h->device));
     return launch_observe(h, "td_observe_as", h->records, h->n_envs, obs_format, obs_dev, stream);
+}
+
+// td_action_mask_kernel over the handle's records
+static int launch_action_mask(td_handle *h, uint8_t *def_mask_dev, uint8_t *atk_mask_dev, void *stream)
+{
+    StepParams p;
+    fill_params(h, p);
+    void *args[] = {&p, &def_mask_dev, &atk_mask_dev};
+    const cudaError_t e = cudaLaunchKernel(action_mask_kernel(h->L), dim3(grid_of(h)), dim3(kWarpsPerCta * 32), args,
+                                           mask_smem_of(h), (cudaStream_t)stream);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(h, TD_E_CUDA, std::string("td_action_mask: ") + cudaGetErrorString(e));
+    }
+    return TD_OK;
+}
+
+extern "C" int td_action_mask(td_handle *h, uint8_t *def_mask_dev, uint8_t *atk_mask_dev, void *stream)
+{
+    if (!h) return TD_E_INVALID;
+    if (!def_mask_dev && !atk_mask_dev) return fail(h, TD_E_INVALID, "td_action_mask: both masks are NULL");
+    if (def_mask_dev && h->kind == TD_KIND_ATK)
+        return fail(h, TD_E_INVALID, "td_action_mask: the attacker env has no defender mask (its defender is scripted)");
+    if (atk_mask_dev && h->kind == TD_KIND_DEF)
+        return fail(h, TD_E_INVALID, "td_action_mask: the defender env has no attacker mask (its attacker is scripted)");
+    if (h->n_maps < 1) return fail(h, TD_E_STATE, "td_action_mask: upload maps and reset first");
+    TD_CUDA(h, cudaSetDevice(h->device));
+    return launch_action_mask(h, def_mask_dev, atk_mask_dev, stream);
 }
 
 // Compact snapshots (SURVEY 8(f) f4): the env records as they are, and observations rebuilt from them later.

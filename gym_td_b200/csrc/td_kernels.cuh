@@ -350,6 +350,103 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) td_observe_kernel(const __g
     write_obs(w, obs + (size_t)env * TD_NCHANNELS * w.ncells());
 }
 
+// Action masks (td_action_mask): which defender actions and attacker summons the next step would carry out, decided
+// from the env record by the legality predicates of td_rules.cuh.  The warp reads only what they need, into a slice
+//   [ td_env_header 64 | map6 cells_pad | MapHdr 16 | towers 32 x 16 | per-cell table cells_pad ]
+// (map6 and the MapHdr are adjacent in the record as well), not the generator words, enemies or static planes.
+__host__ __device__ constexpr int mask_smem_per_warp(int cells_pad)
+{
+    return (int)sizeof(td_env_header) + cells_pad + kMapHdrBytes + TD_CAP_TOWERS * kTowerBytes + cells_pad;
+}
+
+// def_mask: [n, 6 cells + 1] bytes, entry a = 1 when the Discrete action a would come back as RealAction a (the
+// first 6 cells are the (6, L, L) layout of the multi-action Box, one flag each).  atk_mask: [n, 3, 4] bytes, entry
+// (r, t) = 1 when a cluster whose only slot is type t on road r would summon it.  Either may be NULL.
+template <int CELLS>
+__global__ void __launch_bounds__(kWarpsPerCta * 32)
+td_action_mask_kernel(const __grid_constant__ StepParams p, uint8_t *def_mask, uint8_t *atk_mask)
+{
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int env = blockIdx.x * kWarpsPerCta + warp;
+    if (env >= p.n_envs) return;
+    const DevConfig &cc = p.cfg;
+    const int cells = CELLS > 0 ? CELLS : p.cells, cells_pad = CELLS > 0 ? ((CELLS + 15) & ~15) : p.cells_pad;
+    uint8_t *slice = td_smem + (size_t)warp * mask_smem_per_warp(cells_pad);
+    const td_env_header *hdr = reinterpret_cast<const td_env_header *>(slice);
+    uint8_t *map6 = slice + sizeof(td_env_header);
+    const MapHdr *mh = reinterpret_cast<const MapHdr *>(map6 + cells_pad);
+    const td_tower_rec *tw = reinterpret_cast<const td_tower_rec *>(map6 + cells_pad + kMapHdrBytes);
+    uint8_t *table = map6 + cells_pad + kMapHdrBytes + TD_CAP_TOWERS * kTowerBytes;
+    const uint8_t *rec = p.records + (size_t)env * p.record_bytes;
+
+    // header, then map6 + MapHdr (only the MapHdr without a defender mask): one round trip
+    async_copy16(slice, rec, (int)sizeof(td_env_header) >> 4, lane);
+    if (def_mask) async_copy16(map6, rec + p.off_static - cells_pad, (cells_pad + kMapHdrBytes) >> 4, lane);
+    else async_copy16(map6 + cells_pad, rec + p.off_static, kMapHdrBytes >> 4, lane);
+    async_wait_all();
+
+    if (def_mask) {
+        const double cost_def = hdr->cost_def;
+        const int nt = hdr->n_towers;
+        async_copy16(const_cast<td_tower_rec *>(tw), rec + p.off_towers, nt, lane);
+        for (int q = lane; q < (cells_pad >> 2); q += kLanes) reinterpret_cast<uint32_t *>(table)[q] = 0u;
+        async_wait_all();
+        // lane = tower: the first tower of the list on a cell (the one find_tower picks) marks it in the table,
+        // bit 0 = a tower stands there (Destruct), bit 1 = its LvUp succeeds
+        static_assert(TD_CAP_TOWERS == kLanes, "one tower per lane");
+        const bool have = lane < nt;
+        const int loc = have ? tw[lane].loc : 0;
+        const unsigned same = __match_any_sync(kFull, have ? (unsigned)loc : 0x10000u + lane);
+        if (have && lane == __ffs(same) - 1) table[loc] = (uint8_t)(1u | (can_lvup(cc, cost_def, tw[lane].type_lv) ? 2u : 0u));
+        __syncwarp();
+        // lane = cell: bit ch of table[cell] = entry (ch, cell), build 0..3, LvUp, Destruct
+        const bool acts = acts_next(hdr->defender_cd);
+        for (int cell = lane; cell < cells; cell += kLanes) {
+            const unsigned tower = table[cell];
+            unsigned bits = 0;
+            if (acts) {
+#pragma unroll
+                for (int t = 0; t < TD_NTYPES; ++t) bits |= (can_build(cc, cost_def, t, map6[cell], nt) ? 1u : 0u) << t;
+                bits |= ((tower >> 1) & 1u) << 4 | (tower & 1u) << 5;
+            }
+            table[cell] = (uint8_t)bits;
+        }
+        __syncwarp();
+        // The row (6 cells + 1 bytes, so rows of successive envs start at every alignment) in 16-byte chunks of the
+        // aligned address space: whole chunks go out in one store, the partial chunks at either end byte by byte.
+        const int row_bytes = 6 * cells + 1;
+        uint8_t *row = def_mask + (size_t)env * row_bytes;
+        const int head = (int)(reinterpret_cast<uintptr_t>(row) & 15);
+        const int chunks = (head + row_bytes + 15) >> 4;
+        for (int q = lane; q < chunks; q += kLanes) {
+            const int i0 = 16 * q - head;             // row entry of the chunk's first byte (negative: before the row)
+            int ch = 0, cell = i0;
+            if (i0 > 0) { ch = i0 / cells; cell = i0 - ch * cells; }
+            uint32_t v[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+            for (int j = 0; j < 16; ++j) {
+                const int i = i0 + j;
+                if (i >= 0 && i < row_bytes) v[j >> 2] |= (ch < 6 ? (table[cell] >> ch) & 1u : 1u) << (8 * (j & 3));   // the no-op: always 1
+                if (++cell == cells) { cell = 0; ++ch; }
+            }
+            uint8_t *dst = row - head + 16 * q;
+            if (i0 >= 0 && i0 + 16 <= row_bytes) {
+                *reinterpret_cast<uint4 *>(dst) = make_uint4(v[0], v[1], v[2], v[3]);
+            } else {
+#pragma unroll
+                for (int j = 0; j < 16; ++j)
+                    if (i0 + j >= 0 && i0 + j < row_bytes) dst[j] = (uint8_t)(v[j >> 2] >> (8 * (j & 3)));
+            }
+        }
+    }
+    if (atk_mask && lane < TD_ROADS * TD_NTYPES) {
+        const int r = lane / TD_NTYPES, t = lane % TD_NTYPES;
+        const bool ok = acts_next(hdr->attacker_cd) && r < mh->num_roads &&
+                        can_summon(cc, hdr->cost_atk, t, summon_level(cc, hdr->steps));
+        atk_mask[(size_t)env * TD_ROADS * TD_NTYPES + lane] = ok ? 1 : 0;
+    }
+}
+
 // deterministic reduction of the per-env statistics: one block, fixed order
 __global__ void __launch_bounds__(256) td_stats_kernel(const EnvStats *s, int n, long long steps, td_stats *out)
 {

@@ -7,6 +7,41 @@
 namespace td {
 
 // ------------------------------------------------------------------------------------------------
+// Legality: every test that decides whether a defender operation or a summon succeeds.  The rules below and the
+// action masks (td_action_mask_kernel) both call these, so that a mask says exactly what the next step would do.
+
+// A purse pays a price unless it is smaller: the reference's `if cost < price: fail`, so a NaN or infinite purse
+// or price behaves as it does there.
+__device__ __forceinline__ bool affords(double purse, double price) { return !(purse < price); }
+// a tower may stand on a cell outside every tower's diamond and off the road: map[6] == 0 (TDBoard.py:229)
+__device__ __forceinline__ bool cell_free(uint8_t map6_at) { return map6_at == 0; }
+// the tower list holds TD_CAP_TOWERS towers; a build beyond that fails (and flags the env)
+__device__ __forceinline__ bool tower_room(int nt) { return nt < TD_CAP_TOWERS; }
+__device__ __forceinline__ bool below_max_lv(int lv) { return lv < TD_NLV - 1; }
+// level of the enemies a summon creates: progress >= enemy_upgrade_at, progress = steps / max_steps (TDBoard.py:201)
+__device__ __forceinline__ int summon_level(const DevConfig &cc, int steps) { return steps >= cc.upgrade_step ? 1 : 0; }
+// A player whose header cooldown is `cd` may act in the next step: the step lowers it to max(cd - 1, 0) first
+// (TDDefense.py:38-39), and an operation needs 0.  The same test gives AllowNextMove.
+__device__ __forceinline__ bool acts_next(int cd) { return cd <= 1; }
+
+// building type t on a cell succeeds (tower_build checks cost, then position, then capacity)
+__device__ __forceinline__ bool can_build(const DevConfig &cc, double cost_def, int t, uint8_t map6_at, int nt)
+{
+    return affords(cost_def, cc.tower_cost[t][0]) && cell_free(map6_at) && tower_room(nt);
+}
+// LvUp of the tower with type_lv `tl` succeeds (tower_lvup, once it found the tower)
+__device__ __forceinline__ bool can_lvup(const DevConfig &cc, double cost_def, int tl)
+{
+    const int ty = tl & 3, lv = tl >> 2;
+    return below_max_lv(lv) && affords(cost_def, cc.tower_cost[ty][lv + 1]);
+}
+// a cluster slot of type t summons its enemy at level lv (summon_cluster tests the cheapest type first, then t)
+__device__ __forceinline__ bool can_summon(const DevConfig &cc, double cost_atk, int t, int lv)
+{
+    return affords(cost_atk, cc.min_enemy_cost[lv]) && affords(cost_atk, cc.enemy_cost[t][lv]);
+}
+
+// ------------------------------------------------------------------------------------------------
 // (a) defender operations -- all arguments and results are warp-uniform
 
 // map[6] += delta on the Manhattan diamond around `loc` (TDBoard.py:239-245, 281-287).  Out of line: it is
@@ -35,9 +70,9 @@ __device__ __forceinline__ bool tower_build(W &w, int t, int loc, bool &map6_dir
 {
     const DevConfig &cc = w.pp->cfg;
     const double cost = cc.tower_cost[t][0];
-    if (w.cost_def < cost) { w.fail = TD_FC_COST_SHORTAGE; return false; }
-    if (w.map6()[loc] > 0) { w.fail = TD_FC_INVALID_POSITION; return false; }
-    if (w.nt >= TD_CAP_TOWERS) { w.flags |= 2; w.fail = TD_FC_INVALID_POSITION; return false; }
+    if (!affords(w.cost_def, cost)) { w.fail = TD_FC_COST_SHORTAGE; return false; }
+    if (!cell_free(w.map6()[loc])) { w.fail = TD_FC_INVALID_POSITION; return false; }
+    if (!tower_room(w.nt)) { w.flags |= 2; w.fail = TD_FC_INVALID_POSITION; return false; }
     TD_CHECK(w, loc >= 0 && loc < w.ncells() && t >= 0 && t < TD_NTYPES);
     if (w.lane == 0) {
         td_tower_rec &r = w.tw()[w.nt];
@@ -72,9 +107,9 @@ __device__ __forceinline__ bool tower_lvup(W &w, int loc)                       
     int idx = find_tower(w, loc);
     if (idx < 0) { w.fail = TD_FC_UNKNOWN_TARGET; return false; }
     int tl = w.tw()[idx].type_lv, ty = tl & 3, lv = tl >> 2;
-    if (lv >= TD_NLV - 1) { w.fail = TD_FC_LV_MAX; return false; }
+    if (!below_max_lv(lv)) { w.fail = TD_FC_LV_MAX; return false; }
     const double cost = cc.tower_cost[ty][lv + 1];
-    if (w.cost_def < cost) { w.fail = TD_FC_COST_SHORTAGE; return false; }
+    if (!affords(w.cost_def, cost)) { w.fail = TD_FC_COST_SHORTAGE; return false; }
     __syncwarp();
     if (w.lane == 0) w.tw()[idx].type_lv = (uint8_t)(ty | ((lv + 1) << 2));
     __syncwarp();
@@ -168,10 +203,10 @@ __device__ __forceinline__ void decode_multi(W &w, const long long *act, long lo
                 bool can = false;
                 if (flags) {
                     if (tower_at[cell]) can = (flags & 0x30u) != 0 || false;
-                    if (!can && (flags & 0x0fu) && w.map6()[cell] == 0) {
+                    if (!can && (flags & 0x0fu) && cell_free(w.map6()[cell])) {
 #pragma unroll
                         for (int t = 0; t < TD_NTYPES; ++t)
-                            can = can || (((flags >> t) & 1u) && !(w.cost_def < cc.tower_cost[t][0]));
+                            can = can || (((flags >> t) & 1u) && affords(w.cost_def, cc.tower_cost[t][0]));
                     }
                     // a flagged build on a free cell can create the tower that a flagged LvUp/destruct then hits
                 }
@@ -227,7 +262,7 @@ __device__ __forceinline__ bool summon_cluster(W &w, int road, long long &mine, 
 {
     const DevConfig &cc = w.pp->cfg;
     const int start = w.mh()->start[road];
-    const int lv = w.steps >= cc.upgrade_step ? 1 : 0;      // progress >= enemy_upgrade_at
+    const int lv = summon_level(cc, w.steps);
     const int tv = (mine < 0 || mine >= TD_NTYPES) ? TD_NTYPES : (int)mine;     // 4 == enemy_types: empty slot
     const unsigned b0 = __ballot_sync(kFull, tv & 1) >> lane_base, b1 = __ballot_sync(kFull, tv & 2) >> lane_base,
                    b2 = __ballot_sync(kFull, tv & 4) >> lane_base;
@@ -236,12 +271,12 @@ __device__ __forceinline__ bool summon_cluster(W &w, int road, long long &mine, 
     unsigned ok = 0, poor = 0;
     const double cheapest = cc.min_enemy_cost[lv];
     while (todo) {
-        if (w.cost_atk < cheapest) { poor |= todo; break; }      // an empty purse fails every remaining slot alike
+        if (!affords(w.cost_atk, cheapest)) { poor |= todo; break; }      // an empty purse fails every remaining slot alike
         const int k = __ffs(todo) - 1;
         todo &= todo - 1;
         const int t = ((b0 >> k) & 1) | (((b1 >> k) & 1) << 1);
         const double cost = cc.enemy_cost[t][lv];
-        if (w.cost_atk < cost) poor |= 1u << k;
+        if (!affords(w.cost_atk, cost)) poor |= 1u << k;
         else { w.cost_atk = __dsub_rn(w.cost_atk, cost); ok |= 1u << k; }
     }
     int n = __popc(ok);
@@ -274,12 +309,12 @@ __device__ __forceinline__ void summon_uniform(W &w, int t, int road)
 {
     const DevConfig &cc = w.pp->cfg;
     const int start = w.mh()->start[road];
-    const int lv = w.steps >= cc.upgrade_step ? 1 : 0;      // progress >= enemy_upgrade_at
+    const int lv = summon_level(cc, w.steps);
     const double cost = cc.enemy_cost[t][lv];
     int n = 0;
 #pragma unroll 1
     for (int k = 0; k < TD_CLUSTER; ++k) {
-        if (w.cost_atk < cost) break;
+        if (!affords(w.cost_atk, cost)) break;
         w.cost_atk = __dsub_rn(w.cost_atk, cost);
         ++n;
     }

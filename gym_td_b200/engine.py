@@ -96,7 +96,7 @@ EXPORTS = ["td_abi_version", "td_last_error", "td_default_config", "td_mapgen", 
            "td_seed_opponent", "td_set_difficulty", "td_step", "td_observe", "td_step_host", "td_get_state",
            "td_set_state", "td_get_opponent", "td_get_stats", "td_reset_stats", "td_rollout_mask", "td_rollout_record",
            "td_gae", "td_snapshot", "td_observe_snapshot", "td_set_option", "td_packed_stride", "td_invalidate_obs", "td_observe_as",
-           "td_alloc_compressible", "td_free_compressible", "td_upgrade_step"]
+           "td_alloc_compressible", "td_free_compressible", "td_upgrade_step", "td_action_mask"]
 
 
 def lib():
@@ -144,6 +144,7 @@ def lib():
         L.td_alloc_compressible.argtypes = [C.c_int, C.c_size_t, C.c_void_p, C.c_void_p]
         L.td_free_compressible.argtypes = [C.c_void_p]
         L.td_upgrade_step.argtypes = [C.c_int, C.c_double]
+        L.td_action_mask.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         if L.td_abi_version() != 3:
             raise ImportError("libtd_b200.so ABI version mismatch")
         _lib = L
@@ -359,6 +360,12 @@ class Engine(object):
     def observe(self, obs, stream=0, obs_format="f32"):
         fmt = OBS_FORMATS[obs_format] if isinstance(obs_format, str) else int(obs_format)
         self._check(self._lib.td_observe_as(self._h, fmt, _ptr(obs), stream))
+
+    def action_mask(self, def_mask=None, atk_mask=None, stream=0):
+        """td_action_mask: which actions the next step would carry out, from the current env records.  def_mask:
+        uint8 [n, 6*L*L + 1] (TD-def, TD-2p), atk_mask: uint8 [n, 3, 4] (TD-atk, TD-2p); device buffers, either
+        may be None, not both."""
+        self._check(self._lib.td_action_mask(self._h, _ptr(def_mask), _ptr(atk_mask), stream))
 
     # -- state / statistics ---------------------------------------------------------------------
     def get_state_raw(self, first_env=0, n=None):

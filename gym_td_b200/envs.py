@@ -138,6 +138,22 @@ class TDGymBasic(object):
     def step(self, action):
         raise NotImplementedError()
 
+    def action_mask(self):
+        """Which actions the next step() would carry out (TDVecEnv.action_mask for this one env), as numpy bool
+        arrays: TDDefense the Discrete mask [6*L*L + 1] or, with allow_multiple_actions, the single-flag Box mask
+        (6, L, L); TDAttack (3, 4) per (road, enemy type); TDMulti {"Attacker": ..., "Defender": ...}."""
+        L = self.map_size
+        d = torch.zeros((1, 6 * L * L + 1), dtype=torch.uint8, device=self._device) if self._kind != "atk" else None
+        a = torch.zeros((1, E.ROADS, E.NT), dtype=torch.uint8, device=self._device) if self._kind != "def" else None
+        self._engine.action_mask(d, a, self._stream())
+        if d is not None:
+            d = d[0].cpu().numpy().astype(bool)
+            if self._multi():
+                d = d[:-1].reshape(6, L, L)
+        if a is not None:
+            a = a[0].cpu().numpy().astype(bool)
+        return {"def": d, "atk": a, "2p": {"Attacker": a, "Defender": d}}[self._kind]
+
     def render(self, mode="human"):
         raise NotImplementedError("rendering (pyglet viewer, TDBoard.py:387-664) is outside the B200 hot path")
 

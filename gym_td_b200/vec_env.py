@@ -121,6 +121,7 @@ class TDVecEnv(object):
         self._hio_cache = None
         self._host_io = None
         self._host_sig = None
+        self._masks = None
 
     @staticmethod
     def _alloc_bytes(nbytes, dev, mode):
@@ -243,6 +244,28 @@ class TDVecEnv(object):
         """info dict of the last step.  Values are views of the output tensors; the AllowNextMove masks are
         derived from the packed bits only when they are read (no extra kernels on the step path)."""
         return _Info(self)
+
+    def action_mask(self):
+        """Which actions the next step() would carry out, computed on the current stream from the current state
+        (td_action_mask; nothing runs unless this is called).  TD-def: a bool [N, 6*L*L + 1] mask of the Discrete
+        actions, entry a = the action would come back as RealAction a (the no-op is always True); in multi-action mode
+        the [N, 6, L, L] view of its first 6*L*L entries, entry (ch, r, c) = a Box action whose only flag is (ch, r, c)
+        would succeed.  TD-atk: bool [N, 3, 4], entry (road, type) = a cluster whose only slot is that enemy type on
+        that road would summon it (each slot alone: later slots of one cluster see a smaller purse).  TD-2p:
+        {"Attacker": ..., "Defender": ...}.  Views of buffers allocated on the first call, valid until the next call."""
+        N, L = self.num_envs, self.map_size
+        if self._masks is None:
+            self._masks = (torch.zeros((N, 6 * L * L + 1), dtype=torch.uint8, device=self.device) if self.kind != "atk" else None,
+                           torch.zeros((N, E.ROADS, E.NT), dtype=torch.uint8, device=self.device) if self.kind != "def" else None)
+        d, a = self._masks
+        self.engine.action_mask(d, a, torch.cuda.current_stream(self.device).cuda_stream)
+        if d is not None:
+            d = d.view(torch.bool)
+            if self.multi_action:
+                d = d[:, :-1].view(N, 6, L, L)
+        if a is not None:
+            a = a.view(torch.bool)
+        return {"def": d, "atk": a, "2p": {"Attacker": a, "Defender": d}}[self.kind]
 
     # -- host-buffer path (what a numpy-facing gym caller uses) ------------------------------------
     def _host_buffers(self):

@@ -44,7 +44,7 @@ extern "C" {
                               config per handle, td_step_host as one graph launch.  Added since, without a layout
                               change: TD_OPT_GENERIC_KERNELS / HOST_CHAIN / HOST_FIRST_CHUNK / HOST_ZERO_COPY,
                               td_alloc_compressible / td_free_compressible, td_env_header.ep_kills_hi / ep_leaks_hi
-                              in the formerly unused pad2 word */
+                              in the formerly unused pad2 word, td_action_mask */
 
 enum { TD_OK = 0, TD_E_INVALID = -1, TD_E_CUDA = -2, TD_E_ALLOC = -3, TD_E_STATE = -4,
        TD_E_OVERFLOW = -5 };
@@ -288,6 +288,33 @@ int td_invalidate_obs(td_handle *h);
 int td_observe(td_handle *h, float *obs_dev, void *stream);
 /* the same in a reduced-precision element type (TD_OBS_BF16 / TD_OBS_U8; TD_OBS_F32 = td_observe) */
 int td_observe_as(td_handle *h, int obs_format, void *obs_dev, void *stream);
+
+/* Action masks of the current state (new; the reference has none): which actions the NEXT td_step / td_step_host
+ * would carry out.  The state is the one in the env records -- after the last td_step (including its auto-resets),
+ * td_reset or td_set_state -- i.e. the one the current observation shows.  A separate kernel; the step is unchanged.
+ *
+ * def_mask_dev (TD_KIND_DEF, TD_KIND_2P): [n_envs, 6*L*L + 1] uint8, any alignment.  Entry a is 1 exactly when the
+ *   Discrete action a given to the next step comes back with RealAction == a.  So the no-op 6*L*L is always 1, and
+ *   every other entry is 0 unless the defender may act: defender_cd <= 1 in the header (AllowNextMove bit 0; the step
+ *   lowers the cooldown by one before the defender acts).  When it may act, with cost_def the header's purse:
+ *     build type t on loc (a = t*L*L + loc, t < 4):  !(cost_def < tower_cost[t][0]) && map6[loc] == 0
+ *                                                    && n_towers < TD_CAP_TOWERS
+ *     LvUp on loc (a = 4*L*L + loc):                 a tower stands on loc, its level lv is below max_tower_lv
+ *                                                    && !(cost_def < tower_cost[type][lv + 1])
+ *     Destruct on loc (a = 5*L*L + loc):             a tower stands on loc
+ *   (the comparisons are the step's own, so NaN and infinite purses and prices agree with it).  The first 6*L*L
+ *   entries are the channel-major (6, L, L) layout of the multi-action Box: with multi_action, entry (ch, r, c) is 1
+ *   exactly when a Box action whose only flag is (ch, r, c) succeeds (real_def[ch, r, c] == 1).
+ * atk_mask_dev (TD_KIND_ATK, TD_KIND_2P): [n_envs, 3, 4] uint8.  Entry (r, t) is 1 exactly when the next step, given a
+ *   cluster whose only non-empty slot is type t on road r, summons that enemy: attacker_cd <= 1 (AllowNextMove bit 1),
+ *   r < num_roads, and the purse affords the enemy at level lv = (steps >= the upgrade step of td_upgrade_step):
+ *   !(cost_atk < c_min[lv]) && !(cost_atk < enemy_cost[t][lv]), c_min[lv] = the cheapest enemy_cost[.][lv] (the step
+ *   tests the cheapest type first).  A per-slot mask: later slots of one cluster see a smaller purse.  A cluster
+ *   that would exceed the enemy capacity (an error the statistics report as overflow_envs) is not modelled.
+ * In the defender env (TD-def) the defender acts first; in TD-2p the attacker acts first, but a summon changes only
+ * cost_atk and the enemy list, which no defender entry depends on.  Either pointer may be NULL, not both; the mask
+ * of a scripted side (atk mask of TD-def, defender mask of TD-atk) is TD_E_INVALID. */
+int td_action_mask(td_handle *h, uint8_t *def_mask_dev, uint8_t *atk_mask_dev, void *stream);
 
 /* Host-buffer variant (the gym-facing call): copies the actions host->device, steps, copies
  * the small outputs (and the observation if obs_host != NULL) device->host, and synchronises.
